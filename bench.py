@@ -15,6 +15,8 @@ BASELINE.json's north star): ONE recording of T bins split over the ranks; --sca
 every rank holds T bins of an N*T-bin recording.  In strong mode rank 0 also fits the first
 iterations of the same recording alone and the line carries `parity_vs_1rank`.
 --workload nb is configs[2] (decode_latent_naive_bayes only; metric: decode bins/s).
+--dump-outputs DIR writes what the last timed step computed to DIR/<name>.npy (rank 0; the inputs are seeded, so
+two builds run with the same arguments can be compared array for array).
 Prints ONE JSON line on rank 0.
 """
 from __future__ import annotations
@@ -47,6 +49,8 @@ METRIC = "EM time-bins x iters/s"
 UNIT = "bins*iters/s"
 NB_METRIC = "decode bins/s (decode_latent_naive_bayes)"
 NCU_SUMMARY = "profiles/r02_ncu_full_summary.csv"
+DUMP_LIMIT = 64 * 10 ** 6          # bytes written by --dump-outputs in all
+DUMP_TIME_BUDGET = 48 * 10 ** 6    # of which the T-sized arrays (row sample); the rest: tuning, weights, histories
 
 
 def peaks():
@@ -137,6 +141,30 @@ class ClockSampler:
                 "samples": len(sm), "samples_outside_timed_region": n_all - len(sm), "reasons": sorted(reasons)}
 
 
+def dump_rows(T, row_bytes):
+    """Time bins kept by --dump-outputs: all of them when the T-sized arrays fit DUMP_TIME_BUDGET, otherwise a
+    sorted draw without replacement from a fixed seed (the same bins for every build at the same T)."""
+    n = DUMP_TIME_BUDGET // max(1, row_bytes)
+    if T <= n:
+        return np.arange(T)
+    return np.sort(np.random.default_rng(0).choice(T, size=n, replace=False))
+
+
+def write_dump(out_dir, arrays):
+    """name -> tensor / array / scalar, written as out_dir/<name>.npy; float32 stays float32, everything else is
+    stored as float64 (exact for the iteration counts and bin indices)."""
+    host = {}
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if hasattr(a, "detach") else np.asarray(a)
+        host[name] = a if a.dtype == np.float32 else a.astype(np.float64)
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------
 # reference arm: the restated reference (oracle/ref_numpy.py, fp32, reference operation order) on the host
 # ------------------------------------------------------------------------------------------------
@@ -219,7 +247,9 @@ def run_reference(args):
     N, K, T, ls, mv = WORKLOADS[args.workload]
     if args.workload == "nb":
         sample_T = args.cpu_sample_bins or 400
-        rates = [cpu_nb_rate(N, K, sample_T)[0] for _ in range(max(1, min(args.steps, 5)))]
+        for _ in range(args.warmup):
+            cpu_nb_rate(N, K, sample_T)
+        rates = [cpu_nb_rate(N, K, sample_T)[0] for _ in range(args.steps)]
         rate = float(np.median(rates))
         line = {"impl": "reference", "metric": NB_METRIC, "value": rate, "unit": "bins/s", "n_gpus": args.gpus,
                 "steps": args.steps, "warmup": args.warmup, "ms_per_step": sample_T / rate * 1e3,
@@ -360,6 +390,13 @@ def run_nb(args):
     clocks = sampler.stop(wall0, wall1) if rank == 0 else None
     ms = ev0.elapsed_time(ev1)
     launches = ops.LAUNCHES - l0
+    if args.dump_outputs and rank == 0:
+        # the decode of the last timed step (this rank's block); T-sized arrays on a fixed sample of bins
+        rows = dump_rows(Tr, 4 * (3 * K + 1))
+        idx = torch.from_numpy(rows).to(dev)
+        dump = {k: (v.index_select(0, idx) if torch.is_tensor(v) else v) for k, v in out.items()}
+        dump["bins"] = rows
+        write_dump(args.dump_outputs, dump)
     del out
     # end to end: host spikes in, argmax decode + posterior out (the arrays a user reads), median of 3
     y_host = y_dev.cpu().numpy()
@@ -542,6 +579,21 @@ def run_ours(args):
         d = (tu != ref_t).sum().to(torch.float32).reshape(1)
         shard.allreduce_flat_sum_(d)
         tuning_identical = bool(d.item() == 0)
+    if args.dump_outputs and rank == 0:
+        # what the last timed iteration handed its caller: its M-step (tuning, the GLM weights behind it, the Adam
+        # record) and its E-step (log marginal, latent posterior of this rank's block on a fixed sample of bins)
+        n_it = int(m_res[2].item())
+        rows = dump_rows(T_rank, 4 * K)
+        idx = torch.from_numpy(rows).to(dev)
+        if res.gamma_lat is not None:
+            post = res.gamma_lat.index_select(0, idx)
+        else:       # tensor-core statistics: the posterior is kept as fp16 hi/lo pieces (ops.new_gamma16)
+            g = loop.gamma16[:, loop.es.core, :K].index_select(1, idx)
+            post = g[0].float() + g[1].float()
+        write_dump(args.dump_outputs, {
+            "tuning": m_res[4], "params": loop.W_iter, "log_marginal": res.log_marginal,
+            "m_step_n_iter": n_it, "m_step_final": m_res[3], "m_step_loss_history": m_res[0][:n_it],
+            "m_step_error_history": m_res[1][:n_it], "posterior_latent_marg": post, "posterior_bins": rows})
     # Per-phase CUDA events are taken in a SECOND pass of the same number of EM iterations, outside the timed
     # region, with the launching thread synchronising at every mark (each phase timed alone).  Events inside the
     # free-running loop perturb it (an event recorded between the cooperative M-step launch and the next launch
@@ -745,7 +797,14 @@ def main():
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--phase-steps", type=int, default=None,
                     help="EM iterations of the instrumented (per-phase events) pass after the timed region")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step to DIR/<name>.npy (float32/float64, at most "
+                         "64 MB: T-sized arrays on a fixed, seeded sample of time bins, listed in *bins.npy)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of the GPU path (--impl ours)")
     ClockSampler.PERIOD_MS = max(5, args.clocks_ms)
     if args.impl == "reference":
         run_reference(args)

@@ -191,6 +191,28 @@ def test_clock_sampler_parses_nvidia_smi_lines():
     assert abs(out["sm_mhz"] - 1882.5) < 1e-6
 
 
+def test_bench_dump_sample_and_format(tmp_path):
+    """--dump-outputs: a fixed, sorted sample of distinct bins within the budget (all bins when they fit), float32
+    kept, everything else stored as float64, and the 64 MB limit enforced before anything is written."""
+    import importlib.util
+    import torch
+    spec = importlib.util.spec_from_file_location("bench_mod3", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    rows = bench.dump_rows(10 ** 6, 4 * 400)
+    assert len(rows) == bench.DUMP_TIME_BUDGET // 1600 and np.array_equal(rows, bench.dump_rows(10 ** 6, 1600))
+    assert np.all(np.diff(rows) > 0) and rows[0] >= 0 and rows[-1] < 10 ** 6
+    assert np.array_equal(bench.dump_rows(1000, 1600), np.arange(1000))
+    bench.write_dump(str(tmp_path / "d"), {"a": torch.ones(3, 2), "n": 5, "h": torch.tensor(1.5, dtype=torch.float16),
+                                           "bins": rows[:4]})
+    got = {f[:-4]: np.load(tmp_path / "d" / f) for f in os.listdir(tmp_path / "d")}
+    assert set(got) == {"a", "n", "h", "bins"} and got["a"].dtype == np.float32 and got["a"].shape == (3, 2)
+    assert got["n"].dtype == got["h"].dtype == got["bins"].dtype == np.float64 and float(got["h"]) == 1.5
+    with pytest.raises(RuntimeError):
+        bench.write_dump(str(tmp_path / "big"), {"x": np.zeros(bench.DUMP_LIMIT // 4 + 1, np.float32)})
+    assert not (tmp_path / "big").exists()
+
+
 def test_host_buffers_prefault_and_hand_out_arrays():
     """Result buffers are allocated up front and their pages populated on background threads (madvise pieces,
     memset fallback); take() returns the planned array once its pages are in, or None for an unplanned shape."""
