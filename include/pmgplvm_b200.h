@@ -88,6 +88,15 @@ int pmg_counts_to_f16(int64_t T, int N, const float* y, int64_t ldy, void* y16, 
 int pmg_counts_prepare(int64_t T, int N, const float* y, int64_t ldy, const float* ma_neuron, void* y16,
                        int64_t ld16, int ones_col, int* inexact_count, float* lgam, float* ysum,
                        pmg_stream_t stream);
+/* Shuffle tests (reference test.py:22-23, np.roll per neuron): the fp16 operand and lgam of pmg_counts_prepare
+ * (ones_col = 0) for n_shift circular shuffles stacked along time,
+ *   y16[b*T + t, n] = y[(t - shifts[b*N + n]) mod T, n],   lgam[b*T + t] = sum_n m_n lgamma(y16[b*T + t, n] + 1),
+ * bit-identical to pmg_counts_prepare run on each rolled fp32 matrix.  Source: the fp16-exact counts in NEURON-MAJOR
+ * layout yT16 [N, ld_src] (a neuron's shifted window is contiguous).  Out: y16 [n_shift*T, ld16] fp16 (zero padding
+ * from column N), lgam [n_shift*T].  shifts: device int32 [n_shift, N], each in [0, T).  ma_neuron: NULL or [N].
+ * No exactness counter: a circular shift does not change the set of values of a column. */
+int pmg_counts_prepare_shifted(int64_t T, int N, int n_shift, const void* yT16, int64_t ld_src, const int* shifts,
+                               const float* ma_neuron, void* y16, int64_t ld16, float* lgam, pmg_stream_t stream);
 int pmg_emission_tile_n(int K);
 int pmg_emission_prepare_f16(int K, int N, const float* tuning, const float* ma_neuron, float dt, int Kpad,
                              int64_t ld16, void* loglam16, float* lam_sum, pmg_stream_t stream);
@@ -104,6 +113,8 @@ int pmg_naive_bayes_normalize(int64_t T, int K, const float* ll, int64_t ldll, f
 /* same, also writing post = exp(log_post) ([T, ldp]; core.py:517) in the one pass over the rows */
 int pmg_naive_bayes_posterior(int64_t T, int K, const float* ll, int64_t ldll, float* log_post, float* post,
                               int64_t ldp, float* lml_t, pmg_stream_t stream);
+/* lml_t alone (a read-only pass over ll), bit-identical to the lml_t of the two entries above */
+int pmg_naive_bayes_lml(int64_t T, int K, const float* ll, int64_t ldll, float* lml_t, pmg_stream_t stream);
 
 /* ------------------------------------------------------------- F1/F2, S1-S3 --
  * Forward filter (decoder.py:151-198) and backward smoother (decoder.py:200-332)

@@ -49,6 +49,8 @@ SIGNATURES = {
                                         C.c_float, c_f32p, c_f32p, C.c_int64, c_stream]),
     "pmg_counts_prepare": (C.c_int, [C.c_int64, C.c_int, c_f32p, C.c_int64, c_f32p, C.c_void_p, C.c_int64, C.c_int,
                                      c_i32p, c_f32p, c_f32p, c_stream]),
+    "pmg_counts_prepare_shifted": (C.c_int, [C.c_int64, C.c_int, C.c_int, C.c_void_p, C.c_int64, c_i32p, c_f32p,
+                                             C.c_void_p, C.c_int64, c_f32p, c_stream]),
     "pmg_counts_to_f16": (C.c_int, [C.c_int64, C.c_int, c_f32p, C.c_int64, C.c_void_p, C.c_int64, c_i32p, c_stream]),
     "pmg_emission_tile_n": (C.c_int, [C.c_int]),
     "pmg_emission_prepare_f16": (C.c_int, [C.c_int, C.c_int, c_f32p, c_f32p, C.c_float, C.c_int, C.c_int64,
@@ -57,6 +59,7 @@ SIGNATURES = {
                                            c_f32p, c_f32p, c_f32p, c_f32p, C.c_int64, c_stream]),
     "pmg_naive_bayes_normalize": (C.c_int, [C.c_int64, C.c_int, c_f32p, C.c_int64, c_f32p, C.c_int64, c_f32p,
                                             c_stream]),
+    "pmg_naive_bayes_lml": (C.c_int, [C.c_int64, C.c_int, c_f32p, C.c_int64, c_f32p, c_stream]),
     "pmg_naive_bayes_posterior": (C.c_int, [C.c_int64, C.c_int, c_f32p, C.c_int64, c_f32p, c_f32p, C.c_int64, c_f32p,
                                             c_stream]),
     "pmg_forward": (C.c_int, [C.POINTER(PmgScanPlan), C.POINTER(PmgTransition), c_f32p, C.c_int64, c_f32p,

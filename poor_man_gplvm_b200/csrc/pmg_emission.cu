@@ -259,6 +259,19 @@ __global__ void __launch_bounds__(256) emission_gaussian_kernel(int64_t T, int N
   }
 }
 
+// logsumexp_k row[k] by one warp (every lane gets the result); shared by both naive-Bayes kernels so that their
+// lml_t agree bit for bit
+__device__ __forceinline__ float nb_row_logsumexp(const float* __restrict__ row, int K, int lane) {
+  float m = -INFINITY;
+  for (int k = lane; k < K; k += 32) m = fmaxf(m, row[k]);
+  m = warp_max(m);
+  if (!(fabsf(m) <= 3.0e38f)) m = 0.f;   // jax logsumexp: non-finite max -> 0
+  float s = 0.f;
+  for (int k = lane; k < K; k += 32) s += expf(row[k] - m);
+  s = warp_sum(s);
+  return logf(s) + m;
+}
+
 // one warp per time bin: lml = logsumexp_k ll, log_post = ll - lml
 __global__ void nb_normalize_kernel(int64_t T, int K, const float* __restrict__ ll, int64_t ldll,
                                     float* __restrict__ log_post, int64_t ldp, float* __restrict__ lml_t,
@@ -267,14 +280,7 @@ __global__ void nb_normalize_kernel(int64_t T, int K, const float* __restrict__ 
   if (t >= T) return;
   const int lane = threadIdx.x & 31;
   const float* row = ll + (size_t)t * ldll;
-  float m = -INFINITY;
-  for (int k = lane; k < K; k += 32) m = fmaxf(m, row[k]);
-  m = warp_max(m);
-  if (!(fabsf(m) <= 3.0e38f)) m = 0.f;   // jax logsumexp: non-finite max -> 0
-  float s = 0.f;
-  for (int k = lane; k < K; k += 32) s += expf(row[k] - m);
-  s = warp_sum(s);
-  const float lml = logf(s) + m;
+  const float lml = nb_row_logsumexp(row, K, lane);
   float* orow = log_post + (size_t)t * ldp;
   float* prow = post ? post + (size_t)t * ldp : nullptr;
   for (int k = lane; k < K; k += 32) {
@@ -282,6 +288,16 @@ __global__ void nb_normalize_kernel(int64_t T, int K, const float* __restrict__ 
     orow[k] = lp;
     if (prow) prow[k] = expf(lp);            // posterior_latent = exp(log_posterior_latent), core.py:517
   }
+  if (lane == 0) lml_t[t] = lml;
+}
+
+// the log marginal alone (shuffle tests read nothing else): a read-only pass over ll
+__global__ void nb_lml_kernel(int64_t T, int K, const float* __restrict__ ll, int64_t ldll,
+                              float* __restrict__ lml_t) {
+  const int64_t t = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (t >= T) return;
+  const int lane = threadIdx.x & 31;
+  const float lml = nb_row_logsumexp(ll + (size_t)t * ldll, K, lane);
   if (lane == 0) lml_t[t] = lml;
 }
 
@@ -352,6 +368,14 @@ extern "C" int pmg_naive_bayes_normalize(int64_t T, int K, const float* ll, int6
   if (T <= 0 || K <= 0 || !ll || !log_post || !lml_t || ldll < K || ldp < K) return PMG_ERR_BAD_ARG;
   pmg::nb_normalize_kernel<<<pmg::cdiv(T, 8), 256, 0, (cudaStream_t)stream>>>(T, K, ll, ldll, log_post, ldp, lml_t,
                                                                             nullptr);
+  PMG_LAUNCH_CHECK();
+  return PMG_OK;
+}
+
+extern "C" int pmg_naive_bayes_lml(int64_t T, int K, const float* ll, int64_t ldll, float* lml_t,
+                                   pmg_stream_t stream) {
+  if (T <= 0 || K <= 0 || !ll || !lml_t || ldll < K) return PMG_ERR_BAD_ARG;
+  pmg::nb_lml_kernel<<<pmg::cdiv(T, 8), 256, 0, (cudaStream_t)stream>>>(T, K, ll, ldll, lml_t);
   PMG_LAUNCH_CHECK();
   return PMG_OK;
 }

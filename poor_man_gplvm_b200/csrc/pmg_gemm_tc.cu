@@ -128,6 +128,93 @@ counts_prepare_kernel(int64_t T, int N, const float* __restrict__ y, int64_t ldy
   if (__any_sync(0xffffffffu, bad) && lane == 0) atomicAdd(inexact, 1);
 }
 
+// Circularly shifted counts of a shuffle test (np.roll per neuron, reference test.py:22-23), n_shift shuffles stacked
+// along time: y16[b*T + t, n] = yT[n, (t - shifts[b*N + n]) mod T] and lgam[b*T + t] = sum_n m_n lgamma(.+1).
+// The source is neuron-major, so a neuron's shifted window of SH_TT bins is one contiguous (once wrapped) run: a CTA
+// copies the windows of a slab of SH_NS neurons into a time-major shared tile (coalesced along t), then every warp
+// emits SH_TT / 8 rows of it.  lgam reproduces counts_prepare_kernel bit for bit: lane l sums the neurons n with
+// (n >> 2) % 32 == l (VEC, float4 groups) or n % 32 == l, in increasing n, with the same fmaf and the same
+// warp_sum.  SH_NS is a multiple of 128, so that per-lane order survives the slab loop.
+constexpr int SH_TT = 64;                 // output bins per CTA
+constexpr int SH_NS = 256;                // neurons per shared-memory slab
+constexpr int SH_STR = SH_NS + 2;         // tile row stride (halves): 129 words, odd -> conflict-free transpose
+constexpr int SH_THREADS = 256;
+constexpr int SH_RPW = SH_TT / (SH_THREADS / 32);   // rows per warp
+
+template <bool VEC>
+__global__ void __launch_bounds__(SH_THREADS)
+counts_prepare_shifted_kernel(int64_t T, int N, int64_t n_tiles, const __half* __restrict__ yT, int64_t ld_src,
+                              const int* __restrict__ shifts, const float* __restrict__ ma, __half* __restrict__ y16,
+                              int64_t ld16, float* __restrict__ lgam) {
+  __shared__ __align__(16) __half tile[SH_TT * SH_STR];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int64_t b = blockIdx.x / n_tiles;
+  const int64_t t0 = (blockIdx.x - b * n_tiles) * SH_TT;
+  const int* sh = shifts + b * N;
+  float acc[SH_RPW];
+#pragma unroll
+  for (int r = 0; r < SH_RPW; ++r) acc[r] = 0.f;
+  for (int n0 = 0; n0 < N; n0 += SH_NS) {
+    const int ns = min(SH_NS, N - n0);
+    if (n0) __syncthreads();                      // previous slab fully emitted
+    // load: consecutive threads take consecutive bins of one neuron
+    for (int i = threadIdx.x; i < ns * SH_TT; i += SH_THREADS) {
+      const int nl = i / SH_TT, tt = i - nl * SH_TT;
+      const int64_t t = t0 + tt;
+      __half h = __ushort_as_half(0);
+      if (t < T) {
+        int64_t src = t - sh[n0 + nl];
+        if (src < 0) src += T;
+        h = yT[(size_t)(n0 + nl) * ld_src + src];
+      }
+      tile[tt * SH_STR + nl] = h;
+    }
+    __syncthreads();
+#pragma unroll
+    for (int r = 0; r < SH_RPW; ++r) {
+      const int tt = warp * SH_RPW + r;
+      const int64_t t = t0 + tt;
+      if (t >= T) break;
+      const __half* trow = tile + tt * SH_STR;
+      __half* orow = y16 + (size_t)(b * T + t) * ld16 + n0;
+      if (VEC) {
+        for (int jl = lane; jl < (ns >> 2); jl += 32) {
+          const __half2 p0 = *reinterpret_cast<const __half2*>(trow + 4 * jl);
+          const __half2 p1 = *reinterpret_cast<const __half2*>(trow + 4 * jl + 2);
+          const float x[4] = {__low2float(p0), __high2float(p0), __low2float(p1), __high2float(p1)};
+          float m[4] = {1.f, 1.f, 1.f, 1.f};
+          if (ma) {
+            const float4 m4 = __ldg(reinterpret_cast<const float4*>(ma + n0) + jl);
+            m[0] = m4.x; m[1] = m4.y; m[2] = m4.z; m[3] = m4.w;
+          }
+#pragma unroll
+          for (int e = 0; e < 4; ++e) acc[r] = fmaf(m[e], lgamma1p_count(x[e]), acc[r]);
+          uint2 pk;
+          pk.x = *reinterpret_cast<const uint32_t*>(&p0);
+          pk.y = *reinterpret_cast<const uint32_t*>(&p1);
+          reinterpret_cast<uint2*>(orow)[jl] = pk;
+        }
+      } else {
+        for (int nl = lane; nl < ns; nl += 32) {
+          const __half h = trow[nl];
+          const float m = ma ? ma[n0 + nl] : 1.f;
+          acc[r] = fmaf(m, lgamma1p_count(__half2float(h)), acc[r]);
+          orow[nl] = h;
+        }
+      }
+    }
+  }
+#pragma unroll
+  for (int r = 0; r < SH_RPW; ++r) {
+    const int64_t t = t0 + warp * SH_RPW + r;
+    if (t >= T) break;
+    __half* orow = y16 + (size_t)(b * T + t) * ld16;
+    for (int n = N + lane; n < (int)ld16; n += 32) orow[n] = __ushort_as_half(0);
+    const float s = warp_sum(acc[r]);
+    if (lane == 0) lgam[b * T + t] = s;
+  }
+}
+
 // loglam pieces [2][Kpad][ld16]; rows >= K and columns >= N are zero.  One CTA per padded row.
 __global__ void emission_prepare_f16_kernel(int K, int N, const float* __restrict__ tuning,
                                             const float* __restrict__ ma_neuron, float dt, int Kpad, int64_t ld16,
@@ -808,6 +895,28 @@ extern "C" int pmg_counts_prepare(int64_t T, int N, const float* y, int64_t ldy,
   else
     pmg::counts_prepare_kernel<false><<<grid, 256, 0, st>>>(T, N, y, ldy, ma_neuron, (__half*)y16, ld16, ones_col,
                                                             inexact_count, lgam, ysum);
+  PMG_LAUNCH_CHECK();
+  return PMG_OK;
+}
+
+extern "C" int pmg_counts_prepare_shifted(int64_t T, int N, int n_shift, const void* yT16, int64_t ld_src,
+                                          const int* shifts, const float* ma_neuron, void* y16, int64_t ld16,
+                                          float* lgam, pmg_stream_t stream) {
+  if (T <= 0 || N <= 0 || n_shift <= 0 || !yT16 || !shifts || !y16 || !lgam) return PMG_ERR_BAD_ARG;
+  if (ld_src < T || ld16 < N || (ld16 & 7)) return PMG_ERR_BAD_ARG;
+  if ((uintptr_t)y16 & 15) return PMG_ERR_ALIGNMENT;
+  const int64_t n_tiles = (T + pmg::SH_TT - 1) / pmg::SH_TT;
+  if (n_tiles * n_shift > 0x7fffffffLL) return PMG_ERR_UNSUPPORTED_SHAPE;
+  // same float4 / scalar choice as pmg_counts_prepare on a contiguous [T, N] matrix (the lane order of lgam)
+  const bool vec = (N & 3) == 0 && (!ma_neuron || ((uintptr_t)ma_neuron & 15) == 0);
+  const unsigned grid = (unsigned)(n_tiles * n_shift);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (vec)
+    pmg::counts_prepare_shifted_kernel<true><<<grid, pmg::SH_THREADS, 0, st>>>(
+        T, N, n_tiles, (const __half*)yT16, ld_src, shifts, ma_neuron, (__half*)y16, ld16, lgam);
+  else
+    pmg::counts_prepare_shifted_kernel<false><<<grid, pmg::SH_THREADS, 0, st>>>(
+        T, N, n_tiles, (const __half*)yT16, ld_src, shifts, ma_neuron, (__half*)y16, ld16, lgam);
   PMG_LAUNCH_CHECK();
   return PMG_OK;
 }

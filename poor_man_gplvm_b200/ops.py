@@ -158,6 +158,45 @@ class CountsF16:
         return self._exact
 
 
+class CountsF16Shifted:
+    """The fp16 operand and lgamma row term of ``CountsF16(want_lgam=True)`` for ``n_shift`` circular shuffles of the
+    same counts, stacked along time: row ``b*T + t`` holds bin t of shuffle b (np.roll of neuron n by
+    ``shifts[b, n]``).  Same attributes as CountsF16 (``T`` = n_shift * T rows), so the emission GEMM takes it as is;
+    bit-identical to CountsF16 of each rolled fp32 matrix."""
+    ones_col = False
+    exact = True          # a circular shift keeps each neuron's values: exact whenever the unshifted counts are
+
+    def __init__(self, yT16, T, shifts, ld16, ma_vec=None, data=None, lgam=None):
+        """yT16: [N, >=T] fp16, the fp16-exact counts in neuron-major layout; shifts: int32 [n_shift, N] on the
+        device, each in [0, T).  data / lgam: optional buffers of at least n_shift*T rows (views are taken)."""
+        lib = _lib.load()
+        if not (isinstance(yT16, torch.Tensor) and yT16.is_cuda and yT16.dtype == torch.float16 and yT16.dim() == 2
+                and (yT16.stride(1) == 1 or yT16.shape[1] == 1)):
+            raise TypeError("yT16 must be a row-major [N, T] float16 CUDA tensor")
+        self.N = yT16.shape[0]
+        if (not isinstance(shifts, torch.Tensor) or shifts.dtype != torch.int32 or shifts.dim() != 2
+                or shifts.shape[1] != self.N or not shifts.is_contiguous()):
+            raise ValueError("shifts must be a contiguous int32 [n_shift, %d] tensor" % self.N)
+        if yT16.shape[1] < T:
+            raise ValueError("yT16 has %d time bins, fewer than T=%d" % (yT16.shape[1], T))
+        self.n_shift = shifts.shape[0]
+        self.T = self.n_shift * int(T)
+        self.ld = int(ld16)
+        if ma_vec is not None:
+            _f32(ma_vec, "ma_neuron", 1)
+            if ma_vec.shape[0] != self.N:
+                raise ValueError("ma_neuron must be [N]")
+        dev = yT16.device
+        self.data = (torch.empty((self.T, self.ld), dtype=torch.float16, device=dev) if data is None
+                     else data[:self.T])
+        self.lgam = torch.empty(self.T, dtype=torch.float32, device=dev) if lgam is None else lgam[:self.T]
+        self.ysum = None
+        check(lib.pmg_counts_prepare_shifted(int(T), self.N, self.n_shift, _p(yT16), yT16.stride(0), _p(shifts),
+                                             _p(ma_vec), _p(self.data), self.ld, _p(self.lgam), _stream()),
+              "pmg_counts_prepare_shifted")
+        _count(1)
+
+
 def emission_tile_n(K):
     return int(_lib.load().pmg_emission_tile_n(int(K)))
 
@@ -183,6 +222,9 @@ def emission_prepare_f16(tuning, y16, ma_neuron=None, dt=1.0):
                                        _p(lam_sum), _stream()), "pmg_emission_prepare_f16")
     _count(1)
     return L16, lam_sum
+
+
+EMISSION_MAX_ROWS = (1 << 31) - 256     # time bins of one pmg_emission_poisson_f16 call
 
 
 def emission_poisson_f16(y16, L16, lam_sum, lgam, K, ma_latent=None, out=None):
@@ -339,6 +381,20 @@ def naive_bayes_normalize(ll, inplace=False, want_post=False):
           "pmg_naive_bayes_normalize")
     _count(1)
     return log_post, lml
+
+
+def naive_bayes_lml(ll, out=None):
+    """lml_t[T] = logsumexp_k ll[t,:] alone (no log_post write), bit-identical to naive_bayes_normalize's lml_t."""
+    lib = _lib.load()
+    _f32(ll, "ll", 2)
+    T, K = ll.shape
+    if out is None:
+        out = torch.empty(T, dtype=torch.float32, device=ll.device)
+    elif out.dtype != torch.float32 or out.numel() != T or not out.is_contiguous():
+        raise ValueError("out must be a contiguous float32 tensor of %d entries" % T)
+    check(lib.pmg_naive_bayes_lml(T, K, _p(ll), ll.stride(0), _p(out), _stream()), "pmg_naive_bayes_lml")
+    _count(1)
+    return out
 
 
 # ----------------------------------------------------------------------------- transitions
