@@ -230,6 +230,35 @@ int pmg_backward_compact(const pmg_scan_plan* plan, const pmg_transition* tr, co
                          float* beta_halo, float* beta_end, int mode, const int* chain_ids, int n_ids,
                          pmg_stream_t stream);
 
+/* Viterbi decoding (beyond the reference, which returns marginals only): the most probable joint path of the
+ * (dynamics, latent) chain, s = d*K + x, transition M[d,d'] P_{d'}[x,x'] with P_1 = 1/K.  Bin 0's prior is the one
+ * pmg_forward forms from carry_in (the start is marginalised), every later bin takes the max over predecessors;
+ * exact ties go to the smallest flat index d*K + x.  Time-parallel over the chains of pmg_forward.
+ *
+ * pmg_viterbi_forward: plan, transition (kind 0 or 1, any K <= 4096), warm starts (carry_in, warm_in, warm_stride,
+ *   warm_out), mode 0/1/2 and chain_ids exactly as pmg_forward; modes 1 and 2 need warm_in (the carry snapshots).
+ *   Messages are normalised by their sum every bin, as in the filter, so pmg_seam_check_fix applies to them.
+ *   bp:       int16 [T, 2, ldbp] (ldbp >= K): bp[t, d', x'] = flat predecessor state of (d', x') at bin t, written
+ *             for the core bins t > 0 (row 0 is unused);
+ *   lmr:      [T] = log(sum of the unnormalised message) + s*max_k ll[t,k] at the core bins, so that
+ *             log max_path p(path, y) = sum_t lmr[t] + log max(message at the last bin);
+ *   halo_state: [n_chain, 2, K] or NULL, the warmed-up message at t_begin-1 (the seam estimate);
+ *   end_msg:  [n_chain, 2, K] or NULL, the message at each chain's last core bin (the seam truth of the next chain;
+ *             the last one is the message pmg_viterbi_backtrack starts from). */
+int pmg_viterbi_forward(const pmg_scan_plan* plan, const pmg_transition* tr, const float* ll, int64_t ldll,
+                        const float* carry_in, const float* warm_in, int64_t warm_stride, float* warm_out,
+                        void* bp, int64_t ldbp, float* lmr, float* halo_state, float* end_msg, int mode,
+                        const int* chain_ids, int n_ids, pmg_stream_t stream);
+/* maps: device int32 [n_chain, 2K]; maps[c, s] = the state at chain c's first core bin on the best path that ends
+ * in state s at its last core bin (2K threads per chain follow bp through the chain's core). */
+int pmg_viterbi_chain_maps(const pmg_scan_plan* plan, int K, const void* bp, int64_t ldbp, int* maps,
+                           pmg_stream_t stream);
+/* path: device int32 [T] (core bins written), the flat states d*K + x of the MAP path.  Two launches: one CTA takes
+ * the argmax of last_msg [2K] and resolves every chain's end state from the last chain to the first
+ * (s_{b_c} = maps[c, s_{e_c-1}], s_{e_{c-1}-1} = bp[b_c, s_{b_c}]), then every chain fills its core. */
+int pmg_viterbi_backtrack(const pmg_scan_plan* plan, int K, const void* bp, int64_t ldbp, const int* maps,
+                          const float* last_msg, int* path, pmg_stream_t stream);
+
 /* Dense / wide-band move kernels (gp_kernel.py:61-66 custom_transition_kernel; :14-20 with a large
  * movement_variance; BASELINE configs[4]) on the tensor cores: all chains advance in LOCKSTEP, so the n_chain
  * mat-vecs of one time step are one [n_chain x K] . [K x K] GEMM (tcgen05 kind::f16, both operands as two fp16

@@ -23,6 +23,7 @@ from . import hostio
 from . import jaxprng
 from . import ops
 from . import estep
+from . import viterbi
 from .estep import EStep
 from .shard import TimeShard
 
@@ -40,6 +41,16 @@ def _rewrap_tsd(arr, t_l):
     try:
         import pynapple as nap   # optional; only when the caller handed us a TsdFrame
         return nap.TsdFrame(d=arr, t=t_l)
+    except Exception:
+        return arr
+
+
+def _rewrap_tsd_1d(arr, t_l):
+    if t_l is None:
+        return arr
+    try:
+        import pynapple as nap   # optional; only when the caller handed us a TsdFrame or t_l
+        return nap.Tsd(t=t_l, d=arr)
     except Exception:
         return arr
 
@@ -546,6 +557,64 @@ class PoissonGPLVMJump1D:
                                  "relay_bwd": res.n_relay_bwd, "seam_err_fwd": res.seam_err_fwd,
                                  "seam_err_bwd": res.seam_err_bwd}
         return decoding_res
+
+    def _viterbi_inputs(self, y, ma_neuron, ma_latent):
+        """Shape checks of decode_latent_viterbi, on the host before any device work."""
+        shp = tuple(getattr(y, "shape", np.shape(y)))
+        if len(shp) != 2 or shp[0] < 1 or shp[1] != self.n_neuron:
+            raise ValueError("y must be [T, n_neuron=%d] with T >= 1, got shape %s" % (self.n_neuron, shp))
+        if ma_neuron is not None:
+            ms = tuple(getattr(ma_neuron, "shape", np.shape(ma_neuron)))
+            if ms not in ((self.n_neuron,), (shp[0], self.n_neuron)):
+                raise ValueError("ma_neuron must be [n_neuron] or [T, n_neuron], got %s" % (ms,))
+        if ma_latent is not None:
+            m = ma_latent.detach().cpu().numpy() if isinstance(ma_latent, torch.Tensor) else np.asarray(ma_latent)
+            if m.shape != (self.n_latent_bin,):
+                raise ValueError("ma_latent must be [n_latent_bin=%d], got %s" % (self.n_latent_bin, m.shape))
+            if not np.any(m != 0):
+                raise ValueError("ma_latent masks every latent bin: no path has nonzero probability")
+
+    def _viterbi(self, y, tuning, hyperparam, ma_neuron, ma_latent, likelihood_scale, carry_in_of):
+        """(flat path [T] int64 on the device, log_joint_map float); carry_in_of(op): the message in front of bin 0."""
+        self._viterbi_inputs(y, ma_neuron, ma_latent)
+        if tuning is None:
+            tuning = self.tuning
+        y_dev = self._dev(y)
+        P, logP, M, logM, op = self._transition_pack(hyperparam)
+        ma_n, ma_l = self._masks(ma_neuron, ma_latent, y_dev.shape[0])
+        es = EStep(y_dev, op, ma_n, ma_l, likelihood_scale, emission_factory=self._emission_factory(hyperparam),
+                   carry_in=carry_in_of(op))
+        res = viterbi.run(es, self._dev(tuning))
+        self._last_estep_info = {"n_chain": res.n_chain, "fix_fwd": res.n_fix, "relay_fwd": res.n_relay,
+                                 "seam_err_fwd": res.seam_err}
+        return res.path.to(torch.int64), float(res.log_joint_map.item())
+
+    @_on_device
+    def decode_latent_viterbi(self, y, tuning=None, hyperparam={}, ma_neuron=None, ma_latent=None,
+                              likelihood_scale=1., n_time_per_chunk=10000, t_l=None, return_device=False):
+        """Most probable joint (dynamics, latent) path: argmax over paths of p(path, y).  Beyond the reference.
+
+        Joint state s = (d, x), d in {0 move, 1 jump}, x in [0, K); transition M[d,d'] P_{d'}[x,x'] with P_0 the move
+        kernel of the model (RBF Toeplitz or custom band, as in decode_latent) and P_1 = 1/K.  Bin 0's prior is the
+        filter's prior from its carry, so sum over paths of p(path, y) = exp(log_marginal_final) of decode_latent: the
+        start is marginalised, not maximised.  Emission: likelihood_scale * log-likelihood, as in the filter;
+        ma_latent == 0 bins have likelihood 0 and never lie on the path.  Exact ties resolve to the smallest flat
+        index d*K + x, in every predecessor max and in the final argmax.
+
+        Returns ``map_latent`` and ``map_dynamics`` (int64 [T]; a Tsd when y is a TsdFrame or t_l is given) and
+        ``log_joint_map`` = log p(path*, y).  ``n_time_per_chunk`` is accepted for signature symmetry with
+        decode_latent and ignored (the time-parallel chunking is chosen by the E-step plan; the path does not depend
+        on it beyond the seam tolerance).  ma_neuron: [N] or [T, N].  An ma_latent without a nonzero entry raises
+        ValueError."""
+        y, t_in = _unwrap_tsd(y)
+        if t_in is not None:
+            t_l = t_in
+        path, lj = self._viterbi(y, tuning, hyperparam, ma_neuron, ma_latent, likelihood_scale, lambda op: None)
+        K = self.n_latent_bin
+        conv = (lambda t: t) if return_device else self._host
+        return {'map_latent': _rewrap_tsd_1d(conv(path % K), t_l),
+                'map_dynamics': _rewrap_tsd_1d(conv(path // K), t_l),
+                'log_joint_map': lj}
 
     @_on_device
     def decode_latent_naive_bayes(self, y, tuning=None, hyperparam={}, ma_neuron=None, ma_latent=None,

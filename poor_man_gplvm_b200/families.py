@@ -24,7 +24,9 @@ from . import gp_kernel as gpk
 from . import hostio
 from . import jaxprng
 from . import ops
-from .core import (EMLoop, PoissonGPLVMJump1D, _on_device, _rewrap_tsd, _seed_from_key, _unwrap_tsd)
+from . import viterbi
+from .core import (EMLoop, PoissonGPLVMJump1D, _on_device, _rewrap_tsd, _rewrap_tsd_1d, _seed_from_key,
+                   _unwrap_tsd)
 from .estep import EStep
 
 
@@ -174,12 +176,14 @@ class _GPLVM1DBase(PoissonGPLVMJump1D):
                    carry_in=op.stationary)
         return es, logP
 
-    @staticmethod
-    def _finite(lml):
+    _underflow_msg = ("latent-only filter: the one-step predictive probability underflowed (an observation lies "
+                      "where the smooth prior is zero in fp32); use the jump model for such data")
+
+    @classmethod
+    def _finite(cls, lml):
         v = float(lml)
         if not np.isfinite(v):
-            raise RuntimeError("latent-only filter: the one-step predictive probability underflowed (an observation "
-                               "lies where the smooth prior is zero in fp32); use the jump model for such data")
+            raise RuntimeError(cls._underflow_msg)
         return v
 
     @_on_device
@@ -232,6 +236,25 @@ class _GPLVM1DBase(PoissonGPLVMJump1D):
             res.update({'p_joint_latent': lazy(torch.exp(log_joint)), 'p_transition_latent': lazy(torch.exp(log_trans)),
                         'log_joint_latent': lazy(log_joint), 'log_transition_latent': lazy(log_trans)})
         return res
+
+    @_on_device
+    def decode_latent_viterbi(self, y, tuning=None, hyperparam={}, ma_neuron=None, ma_latent=None,
+                              likelihood_scale=1., n_time_per_chunk=10000, t_l=None, return_device=False):
+        """Most probable latent path argmax p(x_0..x_{T-1}, y) (beyond the reference): the jump model's Viterbi
+        decoding with the degenerate dynamics chain, starting from the uniform latent prior of decode_latent.
+        Returns ``map_latent`` (int64 [T]) and ``log_joint_map``; no ``map_dynamics``.  A bin whose normaliser
+        underflows raises RuntimeError, as in decode_latent."""
+        y, t_in = _unwrap_tsd(y)
+        if t_in is not None:
+            t_l = t_in
+        try:
+            path, lj = self._viterbi(y, tuning, hyperparam, ma_neuron, ma_latent, likelihood_scale,
+                                     lambda op: op.stationary)
+        except viterbi.SeamError as e:      # an underflowed message never matches its neighbour's
+            raise RuntimeError(str(e) + "; " + self._underflow_msg) from e
+        self._finite(lj)
+        conv = (lambda t: t) if return_device else self._host
+        return {'map_latent': _rewrap_tsd_1d(conv(path % self.n_latent_bin), t_l), 'log_joint_map': lj}
 
     def sample_latent(self, T, key=0, movement_variance=1, init_latent=None):
         """reference core.py:206-227 (NumPy stream)."""

@@ -612,6 +612,42 @@ def backward(plan, op, ll, alpha, gamma=None, gamma_lat=None, dyn_marg=None, r_o
     _count(1)
 
 
+def viterbi_bp(T, K, device):
+    """int16 [T, 2, ldbp] backpointer buffer of viterbi_forward (ldbp = K rounded up to 8; rows need no init)."""
+    return torch.empty((T, 2, (K + 7) // 8 * 8), dtype=torch.int16, device=device)
+
+
+def viterbi_forward(plan, op, ll, bp, lmr, halo_state=None, end_msg=None, carry_in=None, mode=0, chain_ids=None,
+                    warm_in=None, warm_out=None, sel_err=None, sel_tol=0.0):
+    """Max-product forward pass with backpointers (pmg_viterbi_forward): pmg_forward's plan, warm-start and repair
+    conventions; bp from viterbi_bp, end_msg [n_chain,2,K] = message at each chain's last core bin."""
+    lib = _lib.load()
+    if bp.dtype != torch.int16 or bp.dim() != 3 or bp.shape[1] != 2 or not bp.is_contiguous():
+        raise ValueError("bp must be a contiguous int16 [T, 2, ldbp] tensor")
+    _select(plan, mode, sel_err, sel_tol)
+    tr = op.cstruct()
+    n_ids = int(chain_ids.numel()) if chain_ids is not None else 0
+    wp, ws = _warm(warm_in)
+    check(lib.pmg_viterbi_forward(C.byref(plan), C.byref(tr), _p(ll), ll.shape[1], _p(carry_in), wp, ws,
+                                  _p(warm_out), _p(bp), bp.shape[2], _p(lmr), _p(halo_state), _p(end_msg), int(mode),
+                                  _p(chain_ids), n_ids, _stream()), "pmg_viterbi_forward")
+    _count(1)
+
+
+def viterbi_chain_maps(plan, K, bp, maps):
+    """maps [n_chain, 2K] int32: state at each chain's first core bin on the best path ending in each state."""
+    check(_lib.load().pmg_viterbi_chain_maps(C.byref(plan), int(K), _p(bp), bp.shape[2], _p(maps), _stream()),
+          "pmg_viterbi_chain_maps")
+    _count(1)
+
+
+def viterbi_backtrack(plan, K, bp, maps, last_msg, path):
+    """path [T] int32 (core bins) = flat states d*K + x of the MAP path ending in argmax(last_msg)."""
+    check(_lib.load().pmg_viterbi_backtrack(C.byref(plan), int(K), _p(bp), bp.shape[2], _p(maps), _p(last_msg),
+                                            _p(path), _stream()), "pmg_viterbi_backtrack")
+    _count(2)
+
+
 def scan_compact_supported(op, likelihood_scale):
     """True when the EM fast path (pmg_forward_compact / pmg_backward_compact) covers this transition."""
     tr = op.cstruct()
