@@ -258,6 +258,21 @@ int pmg_viterbi_chain_maps(const pmg_scan_plan* plan, int K, const void* bp, int
  * (s_{b_c} = maps[c, s_{e_c-1}], s_{e_{c-1}-1} = bp[b_c, s_{b_c}]), then every chain fills its core. */
 int pmg_viterbi_backtrack(const pmg_scan_plan* plan, int K, const void* bp, int64_t ldbp, const int* maps,
                           const float* last_msg, int* path, pmg_stream_t stream);
+/* Time-sharded Viterbi: each rank holds bp for its own core bins (plus halo rows), so the single-device resolve of
+ * pmg_viterbi_backtrack, which walks every chain of the recording, is split in two.
+ * pmg_viterbi_block_link: link, device int32 [2K]; link[s] = the state at bin core_begin - 1 (the left neighbour's last
+ *   core bin) on the best path that ends in state s at core_end - 1.  2K threads each walk the chains from last to
+ *   first (the resolve loop of pmg_viterbi_backtrack, ~2 n_chain dependent loads) and take one more step through
+ *   bp[core_begin]; needs core_begin >= 1 (a rank with a left neighbour).
+ * pmg_viterbi_backtrack_sharded: replaces pmg_viterbi_backtrack on a rank of a time-sharded decode.  gathered: device
+ *   int32 [world][4K + 2], every rank's record in rank order: link [2K] int32 | its last message [2K] fp32 | the fp64
+ *   partial sum of its lmr (two words; not read here).  One CTA takes the argmax of the last rank's message (ties:
+ *   smallest index), follows the links of ranks world-1 .. rank+1 to this rank's end state and resolves the chain end
+ *   states; then every chain fills its core, as in pmg_viterbi_backtrack.  No other collective, no host round trip. */
+int pmg_viterbi_block_link(const pmg_scan_plan* plan, int K, const void* bp, int64_t ldbp, const int* maps, int* link,
+                           pmg_stream_t stream);
+int pmg_viterbi_backtrack_sharded(const pmg_scan_plan* plan, int K, const void* bp, int64_t ldbp, const int* maps,
+                                  const int* gathered, int world, int rank, int* path, pmg_stream_t stream);
 
 /* Dense / wide-band move kernels (gp_kernel.py:61-66 custom_transition_kernel; :14-20 with a large
  * movement_variance; BASELINE configs[4]) on the tensor cores: all chains advance in LOCKSTEP, so the n_chain

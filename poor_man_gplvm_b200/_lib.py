@@ -74,6 +74,10 @@ SIGNATURES = {
                                          c_stream]),
     "pmg_viterbi_backtrack": (C.c_int, [C.POINTER(PmgScanPlan), C.c_int, C.c_void_p, C.c_int64, c_i32p, c_f32p,
                                         c_i32p, c_stream]),
+    "pmg_viterbi_block_link": (C.c_int, [C.POINTER(PmgScanPlan), C.c_int, C.c_void_p, C.c_int64, c_i32p, c_i32p,
+                                         c_stream]),
+    "pmg_viterbi_backtrack_sharded": (C.c_int, [C.POINTER(PmgScanPlan), C.c_int, C.c_void_p, C.c_int64, c_i32p,
+                                                c_i32p, C.c_int, C.c_int, c_i32p, c_stream]),
     "pmg_dense_scan_geometry":(C.c_int, [C.c_int, c_i32p_host, c_i32p_host, c_i32p_host, c_i32p_host]),
     "pmg_dense_scan_workspace_bytes": (C.c_int64, [C.c_int, C.c_int]),
     "pmg_forward_dense": (C.c_int, [C.POINTER(PmgScanPlan), C.POINTER(PmgTransition), C.c_void_p, c_i32p_host,

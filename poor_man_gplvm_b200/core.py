@@ -574,8 +574,10 @@ class PoissonGPLVMJump1D:
             if not np.any(m != 0):
                 raise ValueError("ma_latent masks every latent bin: no path has nonzero probability")
 
-    def _viterbi(self, y, tuning, hyperparam, ma_neuron, ma_latent, likelihood_scale, carry_in_of):
-        """(flat path [T] int64 on the device, log_joint_map float); carry_in_of(op): the message in front of bin 0."""
+    def _viterbi(self, y, tuning, hyperparam, ma_neuron, ma_latent, likelihood_scale, carry_in_of,
+                 time_sharded=False, group=None):
+        """(flat path [T] int64 on the device, log_joint_map float); carry_in_of(op): the message in front of bin 0
+        (time-sharded: in front of rank 0's block; the other ranks' chain 0 starts from the left neighbour)."""
         self._viterbi_inputs(y, ma_neuron, ma_latent)
         if tuning is None:
             tuning = self.tuning
@@ -583,15 +585,16 @@ class PoissonGPLVMJump1D:
         P, logP, M, logM, op = self._transition_pack(hyperparam)
         ma_n, ma_l = self._masks(ma_neuron, ma_latent, y_dev.shape[0])
         es = EStep(y_dev, op, ma_n, ma_l, likelihood_scale, emission_factory=self._emission_factory(hyperparam),
-                   carry_in=carry_in_of(op))
+                   carry_in=carry_in_of(op), shard=TimeShard(group) if time_sharded else None)
         res = viterbi.run(es, self._dev(tuning))
         self._last_estep_info = {"n_chain": res.n_chain, "fix_fwd": res.n_fix, "relay_fwd": res.n_relay,
-                                 "seam_err_fwd": res.seam_err}
+                                 "relay_fwd_boundary": res.n_relay_boundary, "seam_err_fwd": res.seam_err}
         return res.path.to(torch.int64), float(res.log_joint_map.item())
 
     @_on_device
     def decode_latent_viterbi(self, y, tuning=None, hyperparam={}, ma_neuron=None, ma_latent=None,
-                              likelihood_scale=1., n_time_per_chunk=10000, t_l=None, return_device=False):
+                              likelihood_scale=1., n_time_per_chunk=10000, t_l=None, return_device=False,
+                              time_sharded=False, group=None):
         """Most probable joint (dynamics, latent) path: argmax over paths of p(path, y).  Beyond the reference.
 
         Joint state s = (d, x), d in {0 move, 1 jump}, x in [0, K); transition M[d,d'] P_{d'}[x,x'] with P_0 the move
@@ -605,11 +608,16 @@ class PoissonGPLVMJump1D:
         ``log_joint_map`` = log p(path*, y).  ``n_time_per_chunk`` is accepted for signature symmetry with
         decode_latent and ignored (the time-parallel chunking is chosen by the E-step plan; the path does not depend
         on it beyond the seam tolerance).  ma_neuron: [N] or [T, N].  An ma_latent without a nonzero entry raises
-        ValueError."""
+        ValueError.
+
+        time_sharded=True (under torch.distributed, every rank of ``group`` calls together): ``y`` (and a [T, N]
+        ma_neuron) is this rank's contiguous block of bins; ``map_latent`` / ``map_dynamics`` cover that block and
+        ``log_joint_map`` is the global value, identical on every rank.  The path is the single-device path."""
         y, t_in = _unwrap_tsd(y)
         if t_in is not None:
             t_l = t_in
-        path, lj = self._viterbi(y, tuning, hyperparam, ma_neuron, ma_latent, likelihood_scale, lambda op: None)
+        path, lj = self._viterbi(y, tuning, hyperparam, ma_neuron, ma_latent, likelihood_scale, lambda op: None,
+                                 time_sharded, group)
         K = self.n_latent_bin
         conv = (lambda t: t) if return_device else self._host
         return {'map_latent': _rewrap_tsd_1d(conv(path % K), t_l),

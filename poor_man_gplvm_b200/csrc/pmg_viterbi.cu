@@ -9,6 +9,11 @@
 // The backtrack is time-parallel too: pmg_viterbi_chain_maps follows, for every chain and every end state, the
 // backpointers through the chain's core (maps[c, s] = state at the chain's first bin); pmg_viterbi_backtrack then
 // resolves the chain end states from last to first (n_chain dependent lookups) and lets every chain fill its core.
+//
+// Time-sharded runs keep backpointers for the rank's own bins only.  pmg_viterbi_block_link summarises a rank's block
+// as a map from its end state to the left neighbour's end state; the ranks all-gather those maps (with the last
+// messages), and pmg_viterbi_backtrack_sharded resolves this rank's end state from the last rank's argmax before it
+// backtracks its own chains as pmg_viterbi_backtrack does.
 #include <climits>
 
 #include "pmg_common.cuh"
@@ -390,6 +395,10 @@ __global__ void __launch_bounds__(256, 1) viterbi_fwd_kernel(const Params p) {
   }
 }
 
+// words of one rank's record in pmg_viterbi_backtrack_sharded's gathered buffer: link [2K] int32 | last message [2K]
+// fp32 | partial sum of lmr (fp64, two words)
+__host__ __device__ __forceinline__ int64_t viterbi_record_words(int K) { return 4 * (int64_t)K + 2; }
+
 __device__ __forceinline__ int bp_at(const int16_t* bp, int64_t ldbp, int64_t t, int st, int K) {
   const int d = st >= K;
   const int v = __ldg(bp + (size_t)t * 2 * ldbp + (size_t)d * ldbp + (st - d * K));
@@ -410,32 +419,74 @@ __global__ void __launch_bounds__(256) viterbi_maps_kernel(int K, int64_t core_b
   maps[(size_t)c * 2 * K + s0] = st;
 }
 
-// path[e_c - 1] = end state of every chain: argmax of the last message, then chains from last to first
-__global__ void __launch_bounds__(256) viterbi_resolve_kernel(int K, int n_chain, int64_t core_begin,
-                                                              int64_t core_end, int64_t chunk_len, const int16_t* bp,
-                                                              int64_t ldbp, const int* maps, const float* last_msg,
-                                                              int* path) {
+// Chains n_chain-1 .. 0 of a block, from state st at the block's last core bin: path (if given) receives every chain's
+// end state (s_{e_{c-1}-1} = bp[b_c, maps[c, s_{e_c-1}]]).  Returns the state at chain 0's first core bin, or with
+// through_begin the state one bin before it (one more step through bp[core_begin]).
+__device__ int walk_chains(int K, int n_chain, int64_t core_begin, int64_t core_end, int64_t chunk_len,
+                           const int16_t* bp, int64_t ldbp, const int* maps, int st, int* path, bool through_begin) {
+  for (int c = n_chain - 1; c >= 0; --c) {
+    const int64_t b = core_begin + (int64_t)c * chunk_len;
+    const int64_t e = min(b + chunk_len, core_end);
+    if (path) path[e - 1] = st;
+    if (c > 0 || through_begin) st = bp_at(bp, ldbp, b, maps[(size_t)c * 2 * K + st], K);
+  }
+  return st;
+}
+
+// argmax of msg [2K] (ties: smallest index) over the CTA; the result is valid in thread 0
+__device__ int block_argmax(const float* msg, int K) {
   __shared__ float sv[8];
   __shared__ int si[8];
   float bv = -INFINITY;
   int bi = INT_MAX;
   for (int i = threadIdx.x; i < 2 * K; i += blockDim.x) {
-    const float v = last_msg[i];
+    const float v = msg[i];
     if (better(v, i, bv, bi)) { bv = v; bi = i; }
   }
   warp_argmax(bv, bi);
   if ((threadIdx.x & 31) == 0) { sv[threadIdx.x >> 5] = bv; si[threadIdx.x >> 5] = bi; }
   __syncthreads();
-  if (threadIdx.x != 0) return;
   for (int w = 1; w < (int)(blockDim.x >> 5); ++w)
     if (better(sv[w], si[w], bv, bi)) { bv = sv[w]; bi = si[w]; }
-  int st = (unsigned)bi < (unsigned)(2 * K) ? bi : 0;
-  for (int c = n_chain - 1; c >= 0; --c) {
-    const int64_t b = core_begin + (int64_t)c * chunk_len;
-    const int64_t e = min(b + chunk_len, core_end);
-    path[e - 1] = st;
-    if (c > 0) st = bp_at(bp, ldbp, b, maps[(size_t)c * 2 * K + st], K);
+  return (unsigned)bi < (unsigned)(2 * K) ? bi : 0;
+}
+
+// path[e_c - 1] = end state of every chain: argmax of the last message, then chains from last to first
+__global__ void __launch_bounds__(256) viterbi_resolve_kernel(int K, int n_chain, int64_t core_begin,
+                                                              int64_t core_end, int64_t chunk_len, const int16_t* bp,
+                                                              int64_t ldbp, const int* maps, const float* last_msg,
+                                                              int* path) {
+  const int st = block_argmax(last_msg, K);
+  if (threadIdx.x != 0) return;
+  walk_chains(K, n_chain, core_begin, core_end, chunk_len, bp, ldbp, maps, st, path, false);
+}
+
+// link[s] = state at bin core_begin - 1 (the left neighbour rank's last core bin) on the best path that ends in state s
+// at core_end - 1
+__global__ void __launch_bounds__(256) viterbi_link_kernel(int K, int n_chain, int64_t core_begin, int64_t core_end,
+                                                           int64_t chunk_len, const int16_t* bp, int64_t ldbp,
+                                                           const int* maps, int* link) {
+  const int s = blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= 2 * K) return;
+  link[s] = walk_chains(K, n_chain, core_begin, core_end, chunk_len, bp, ldbp, maps, s, nullptr, true);
+}
+
+// time-sharded resolve: argmax of the last rank's last message, the links of ranks world-1 .. rank+1 down to this
+// rank's end state, then this rank's chains as in viterbi_resolve_kernel
+__global__ void __launch_bounds__(256) viterbi_resolve_sharded_kernel(int K, int n_chain, int64_t core_begin,
+                                                                      int64_t core_end, int64_t chunk_len,
+                                                                      const int16_t* bp, int64_t ldbp,
+                                                                      const int* maps, const int* gathered, int world,
+                                                                      int rank, int* path) {
+  const int64_t rec = viterbi_record_words(K);
+  const int* last = gathered + (size_t)(world - 1) * rec;
+  int st = block_argmax((const float*)(last + 2 * K), K);
+  if (threadIdx.x != 0) return;
+  for (int r = world - 1; r > rank; --r) {
+    const int v = gathered[(size_t)r * rec + st];
+    st = (unsigned)v < (unsigned)(2 * K) ? v : 0;
   }
+  walk_chains(K, n_chain, core_begin, core_end, chunk_len, bp, ldbp, maps, st, path, false);
 }
 
 // every chain backtracks its own core from its resolved end state
@@ -536,6 +587,33 @@ extern "C" int pmg_viterbi_backtrack(const pmg_scan_plan* plan, int K, const voi
   pmg::vit::viterbi_resolve_kernel<<<1, 256, 0, st>>>(K, plan->n_chain, plan->core_begin, plan->core_end,
                                                       plan->chunk_len, (const int16_t*)bp, ldbp, maps, last_msg,
                                                       path);
+  PMG_LAUNCH_CHECK();
+  pmg::vit::viterbi_fill_kernel<<<pmg::cdiv(plan->n_chain, 128), 128, 0, st>>>(
+      K, plan->n_chain, plan->core_begin, plan->core_end, plan->chunk_len, (const int16_t*)bp, ldbp, path);
+  PMG_LAUNCH_CHECK();
+  return PMG_OK;
+}
+
+extern "C" int pmg_viterbi_block_link(const pmg_scan_plan* plan, int K, const void* bp, int64_t ldbp, const int* maps,
+                                      int* link, pmg_stream_t stream) {
+  if (!pmg::vit::plan_ok(plan) || plan->core_begin < 1 || !bp || !maps || !link || K <= 0 || K > 4096 || ldbp < K)
+    return PMG_ERR_BAD_ARG;
+  pmg::vit::viterbi_link_kernel<<<pmg::cdiv(2 * K, 256), 256, 0, (cudaStream_t)stream>>>(
+      K, plan->n_chain, plan->core_begin, plan->core_end, plan->chunk_len, (const int16_t*)bp, ldbp, maps, link);
+  PMG_LAUNCH_CHECK();
+  return PMG_OK;
+}
+
+extern "C" int pmg_viterbi_backtrack_sharded(const pmg_scan_plan* plan, int K, const void* bp, int64_t ldbp,
+                                             const int* maps, const int* gathered, int world, int rank, int* path,
+                                             pmg_stream_t stream) {
+  if (!pmg::vit::plan_ok(plan) || !bp || !maps || !gathered || !path || K <= 0 || K > 4096 || ldbp < K ||
+      world < 1 || rank < 0 || rank >= world)
+    return PMG_ERR_BAD_ARG;
+  cudaStream_t st = (cudaStream_t)stream;
+  pmg::vit::viterbi_resolve_sharded_kernel<<<1, 256, 0, st>>>(K, plan->n_chain, plan->core_begin, plan->core_end,
+                                                              plan->chunk_len, (const int16_t*)bp, ldbp, maps,
+                                                              gathered, world, rank, path);
   PMG_LAUNCH_CHECK();
   pmg::vit::viterbi_fill_kernel<<<pmg::cdiv(plan->n_chain, 128), 128, 0, st>>>(
       K, plan->n_chain, plan->core_begin, plan->core_end, plan->chunk_len, (const int16_t*)bp, ldbp, path);

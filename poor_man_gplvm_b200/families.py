@@ -239,17 +239,19 @@ class _GPLVM1DBase(PoissonGPLVMJump1D):
 
     @_on_device
     def decode_latent_viterbi(self, y, tuning=None, hyperparam={}, ma_neuron=None, ma_latent=None,
-                              likelihood_scale=1., n_time_per_chunk=10000, t_l=None, return_device=False):
+                              likelihood_scale=1., n_time_per_chunk=10000, t_l=None, return_device=False,
+                              time_sharded=False, group=None):
         """Most probable latent path argmax p(x_0..x_{T-1}, y) (beyond the reference): the jump model's Viterbi
         decoding with the degenerate dynamics chain, starting from the uniform latent prior of decode_latent.
         Returns ``map_latent`` (int64 [T]) and ``log_joint_map``; no ``map_dynamics``.  A bin whose normaliser
-        underflows raises RuntimeError, as in decode_latent."""
+        underflows raises RuntimeError, as in decode_latent (time-sharded: on every rank, decided from all-reduced
+        data).  time_sharded / group: as in PoissonGPLVMJump1D.decode_latent_viterbi."""
         y, t_in = _unwrap_tsd(y)
         if t_in is not None:
             t_l = t_in
         try:
             path, lj = self._viterbi(y, tuning, hyperparam, ma_neuron, ma_latent, likelihood_scale,
-                                     lambda op: op.stationary)
+                                     lambda op: op.stationary, time_sharded, group)
         except viterbi.SeamError as e:      # an underflowed message never matches its neighbour's
             raise RuntimeError(str(e) + "; " + self._underflow_msg) from e
         self._finite(lj)

@@ -648,6 +648,36 @@ def viterbi_backtrack(plan, K, bp, maps, last_msg, path):
     _count(2)
 
 
+def viterbi_records(n, K, device):
+    """n zeroed records of a time-sharded Viterbi backtrack, int32 [n, 4K + 2] in the layout
+    pmg_viterbi_backtrack_sharded reads: link [2K] int32 | last message [2K] fp32 | partial sum of lmr (fp64)."""
+    return torch.zeros((n, 4 * K + 2), dtype=torch.int32, device=device)
+
+
+def split_viterbi_records(gathered, K):
+    """[n, 4K + 2] int32 records -> (link [n, 2K] int32, msg [n, 2K] fp32, lsum [n] fp64) views."""
+    return (gathered[:, :2 * K], gathered[:, 2 * K:4 * K].view(torch.float32),
+            gathered[:, 4 * K:].view(torch.float64).view(-1))
+
+
+def viterbi_block_link(plan, K, bp, maps, link):
+    """link [2K] int32: state at bin core_begin - 1 on the best path ending in each state at core_end - 1."""
+    check(_lib.load().pmg_viterbi_block_link(C.byref(plan), int(K), _p(bp), bp.shape[2], _p(maps), _p(link),
+                                             _stream()), "pmg_viterbi_block_link")
+    _count(1)
+
+
+def viterbi_backtrack_sharded(plan, K, bp, maps, gathered, rank, path):
+    """path [T] int32 (core bins) of this rank's block of the MAP path; gathered [world, 4K + 2] int32 records."""
+    if gathered.dtype != torch.int32 or gathered.dim() != 2 or gathered.shape[1] != 4 * K + 2 \
+            or not gathered.is_contiguous():
+        raise ValueError("gathered must be contiguous int32 [world, 4K + 2]")
+    check(_lib.load().pmg_viterbi_backtrack_sharded(C.byref(plan), int(K), _p(bp), bp.shape[2], _p(maps),
+                                                    _p(gathered), gathered.shape[0], int(rank), _p(path), _stream()),
+          "pmg_viterbi_backtrack_sharded")
+    _count(2)
+
+
 def scan_compact_supported(op, likelihood_scale):
     """True when the EM fast path (pmg_forward_compact / pmg_backward_compact) covers this transition."""
     tr = op.cstruct()
