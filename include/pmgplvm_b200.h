@@ -385,6 +385,12 @@ int pmg_mstep_adam_ld(int K, int B, int N, const float* Phi, const float* yw, in
                       float* err_hist, int* n_iter_out, float* final_out, float* tuning_out,
                       void* workspace, int64_t workspace_bytes, pmg_stream_t stream);
 
+/* The launch pmg_mstep_adam(_ld) makes for these shapes on the current device, without launching: *kernel = 1 for
+ * the lagged-decision kernel (one neuron tile per CTA, every CTA resident), 0 for the barrier-per-step kernel
+ * (honours PMG_MSTEP_LAG=0 like the launch); *phi_in_smem = 1 when Phi is staged in shared memory; *grid = CTAs;
+ * *parts = parts the gradient's K sum is split into.  Any output may be NULL. */
+int pmg_mstep_plan(int K, int B, int N, int maxiter, int* kernel, int* phi_in_smem, int* grid, int* parts);
+
 /* tuning[k,n] = softplus(sum_b Phi[k,b]*W[b,n])   (fit_tuning_helper.py:11-25) */
 int pmg_tuning_softplus(int K, int B, int N, const float* Phi, const float* W, float* tuning,
                         pmg_stream_t stream);

@@ -161,12 +161,13 @@ def adam_init(params):
 
 
 def adam_run(params, opt_state, param_prior_std, basis, y_weighted, t_weighted,
-             step_size=0.01, maxiter=1000, tol=1e-6, b1=0.9, b2=0.999, eps=1e-8):
+             step_size=0.01, maxiter=1000, tol=1e-6, b1=0.9, b2=0.999, eps=1e-8, min_iters=5):
     """fit_tuning_helper.py:124-196 (make_adam_runner.run).
 
     Loop carried state (i, params, opt_state, error, loss, loss_prev); body runs
-    while ``i < maxiter-1 and (i < 5 or |loss-loss_prev|/max(|loss|,1e-8) > tol)``;
-    ``loss`` lags ``params`` by one update (:168-179).
+    while ``i < maxiter-1 and (i < min_iters or |loss-loss_prev|/max(|loss|,1e-8) > tol)``;
+    ``loss`` lags ``params`` by one update (:168-179).  The reference hard-codes
+    ``min_iters = 5``; the M-step kernels take it as an argument.
     """
     dt = params.dtype
     f = dt.type
@@ -179,7 +180,7 @@ def adam_run(params, opt_state, param_prior_std, basis, y_weighted, t_weighted,
     count, mu, nu = int(opt_state["count"]), opt_state["mu"].copy(), opt_state["nu"].copy()
     while True:
         rel = abs(loss - loss_prev) / max(abs(loss), f(1e-8))
-        if not (i < maxiter - 1 and (i < 5 or rel > f(tol))):
+        if not (i < maxiter - 1 and (i < min_iters or rel > f(tol))):
             break
         new_loss, g = poisson_m_step_value_and_grad(params, param_prior_std, basis, y_weighted, t_weighted)
         mu = f(b1) * mu + f(1 - b1) * g

@@ -131,6 +131,8 @@ SIGNATURES = {
                                     C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.c_int, C.c_float,
                                     C.c_int, c_f32p, c_f32p, c_f32p, c_i32p, c_f32p, c_f32p, c_i32p, c_f32p, c_f32p,
                                     C.c_void_p, C.c_int64, c_stream]),
+    "pmg_mstep_plan": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, c_i32p_host, c_i32p_host, c_i32p_host,
+                                 c_i32p_host]),
     "pmg_threefry_posterior_init": (C.c_int, [C.c_int64, C.c_int, C.c_int64, C.c_int64, C.c_uint32, C.c_uint32,
                                               C.c_float, c_f32p, C.c_int64, c_f32p, C.c_int64, C.c_void_p, C.c_int64,
                                               C.c_int64, C.c_void_p, c_stream]),

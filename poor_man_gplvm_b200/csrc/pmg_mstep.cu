@@ -19,6 +19,9 @@ namespace pmg {
 constexpr int MS_NT = 4;        // neurons per tile
 constexpr int MS_THREADS = 256;
 
+// the gradient phase splits the K rows of Phi into this many parts, one thread per (part, basis function)
+__host__ __device__ constexpr int mstep_parts(int threads, int B) { return B >= threads ? 1 : threads / B; }
+
 struct MstepParams {
   int K, B, N;
   const float* Phi;
@@ -62,7 +65,7 @@ __global__ void __launch_bounds__(MS_THREADS, 1) mstep_adam_kernel(const MstepPa
   float* phiS = smem;                                   // [K][Bs] when phi_in_smem
   float* wS = phiS + (p.phi_in_smem ? (((size_t)K * Bs + 3) & ~(size_t)3) : 0);   // [B][NT], 16B aligned
   float* eS = wS + (size_t)B * MS_NT;                   // [K][NT]
-  const int parts = B >= MS_THREADS ? 1 : MS_THREADS / B;
+  const int parts = mstep_parts(MS_THREADS, B);
   float* gS = eS + (size_t)K * MS_NT;                   // [parts][B][NT]
   __shared__ double redD[2][MS_THREADS / 32];
   __shared__ float bcast[4];
@@ -250,8 +253,11 @@ __global__ void __launch_bounds__(MS_THREADS, 1) mstep_adam_kernel(const MstepPa
 // (per-step slots + per-step arrival counters) and evaluates the reference's stop rule for step i - LAG, by
 // which time all partials of that step have long arrived.  The last LAG+1 optimiser states (W, mu, nu) of the
 // tile live in shared memory; when the rule says "stop before update j", the state after j updates is
-// restored.  Partials, their reduction order and all arithmetic are those of mstep_adam_kernel, so both
-// kernels return the same bits.  One tile per CTA (N <= 4 * #resident CTAs), state of a tile in shared memory.
+// restored.  The per-element arithmetic, the fixed reduction order of the partials and the stop rule are those of
+// mstep_adam_kernel, but with 512 instead of 256 threads the gradient's K sum is split into 512/B instead of 256/B
+// parts and each thread sums the loss over other rows: the two kernels agree to fp32 rounding, not bit for bit.  A
+// rule that rounding cannot decide (tol < 0, a stop at min_iters) stops both at the same step.  One tile per CTA
+// (N <= 4 * #resident CTAs), state of a tile in shared memory.
 // ---------------------------------------------------------------------------------------------------
 constexpr int MS_LAG = 4;        // a step's stop rule is evaluated at least this many steps later
 constexpr int MS_BATCH = 4;      // ... and MS_BATCH steps at a time (one warp per step)
@@ -265,7 +271,7 @@ __global__ void __launch_bounds__(LT, 1) mstep_adam_lag_kernel(const MstepParams
   const int BT = B * MS_NT;
   float* phiS = smem;                                   // [K][Bs] when phi_in_smem
   float* eS = phiS + (p.phi_in_smem ? (((size_t)K * Bs + 3) & ~(size_t)3) : 0);   // [K][NT], 16B aligned
-  const int parts = B >= LT ? 1 : LT / B;
+  const int parts = mstep_parts(LT, B);
   float* gS = eS + (size_t)K * MS_NT;                   // [parts][B][NT]
   float* ywS = gS + (size_t)parts * BT;                 // [K][NT]
   float* twS = ywS + (size_t)K * MS_NT;                 // [K]
@@ -480,7 +486,7 @@ __global__ void __launch_bounds__(LT, 1) mstep_adam_lag_kernel(const MstepParams
 
 template <int LT>
 static size_t mstep_lag_smem(int K, int B, bool phi_in_smem, int Bs) {
-  const int parts = B >= LT ? 1 : LT / B;
+  const int parts = mstep_parts(LT, B);
   size_t f = (size_t)K * MS_NT + (size_t)parts * B * MS_NT + (size_t)K * MS_NT + (size_t)((K + 3) & ~3) +
              (size_t)3 * (MS_LAG + MS_BATCH + 1) * B * MS_NT;
   if (phi_in_smem) f += ((size_t)K * Bs + 3) & ~(size_t)3;
@@ -499,10 +505,65 @@ __global__ void tuning_softplus_kernel(int K, int B, int N, const float* __restr
 }
 
 static size_t mstep_smem(int K, int B, bool phi_in_smem, int Bs) {
-  const int parts = B >= MS_THREADS ? 1 : MS_THREADS / B;
+  const int parts = mstep_parts(MS_THREADS, B);
   size_t f = (size_t)B * MS_NT + (size_t)K * MS_NT + (size_t)parts * B * MS_NT;
   if (phi_in_smem) f += ((size_t)K * Bs + 3) & ~(size_t)3;
   return f * sizeof(float);
+}
+
+constexpr int MS_LAG_THREADS = 512;   // threads per CTA of the lagged kernel (one round over K <= 512 rows of Phi)
+
+struct MstepPlan {
+  int lagged;          // 1: mstep_adam_lag_kernel, 0: mstep_adam_kernel
+  int phi_in_smem, Bs, grid, parts;
+  size_t smem;
+};
+
+// Kernel, placement of Phi and grid of an M-step launch on the current device.  pmg_mstep_adam_ld launches what this
+// returns and pmg_mstep_plan reports it.  Sets the chosen kernel's dynamic shared-memory limit, which the occupancy
+// query and the launch need.
+static int mstep_plan(int K, int B, int N, MstepPlan& pl) {
+  pl.Bs = B | 1;
+  pl.phi_in_smem = mstep_smem(K, B, true, pl.Bs) <= 200 * 1024;
+  pl.smem = mstep_smem(K, B, pl.phi_in_smem, pl.Bs);
+  if (pl.smem > 227 * 1024) return PMG_ERR_UNSUPPORTED_SHAPE;
+  const int ntiles = (N + MS_NT - 1) / MS_NT;
+  int dev = 0, sms = 0;
+  PMG_CUDA_CHECK(cudaGetDevice(&dev));
+  PMG_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  {
+    // lagged-decision kernel: one tile per CTA, all CTAs resident, tile state + operands in shared memory
+    const char* lag_s = std::getenv("PMG_MSTEP_LAG");      // 0 = the barrier-per-step kernel (cross-check)
+    const int lag_env = lag_s ? std::atoi(lag_s) : 1;
+    constexpr int LT = MS_LAG_THREADS;
+    const bool phi_l = mstep_lag_smem<LT>(K, B, true, pl.Bs) <= 200 * 1024;
+    const size_t smem_l = mstep_lag_smem<LT>(K, B, phi_l, pl.Bs);
+    if (lag_env && smem_l <= 200 * 1024) {
+      // attribute + occupancy query once per shared-memory size (host time of a launch that runs every EM iteration)
+      static size_t cached_smem = 0;
+      static int cached_per = 0, cached_dev = -1;
+      if (cached_smem != smem_l || cached_dev != dev) {
+        cached_dev = dev;
+        PMG_CUDA_CHECK(cudaFuncSetAttribute(mstep_adam_lag_kernel<LT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_l));
+        PMG_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&cached_per, mstep_adam_lag_kernel<LT>, LT, smem_l));
+        cached_smem = smem_l;
+      }
+      if (cached_per >= 1 && ntiles <= sms * cached_per && ntiles <= 1024) {
+        pl.lagged = 1; pl.phi_in_smem = phi_l; pl.smem = smem_l; pl.grid = ntiles; pl.parts = mstep_parts(LT, B);
+        return PMG_OK;
+      }
+    }
+  }
+  PMG_CUDA_CHECK(cudaFuncSetAttribute(mstep_adam_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem));
+  int per_sm = 0;
+  PMG_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mstep_adam_kernel, MS_THREADS, pl.smem));
+  if (per_sm < 1) return PMG_ERR_UNSUPPORTED_SHAPE;
+  pl.lagged = 0;
+  pl.grid = sms * per_sm;
+  if (pl.grid > ntiles) pl.grid = ntiles;
+  if (pl.grid > 1024) pl.grid = 1024;
+  pl.parts = mstep_parts(MS_THREADS, B);
+  return PMG_OK;
 }
 
 }  // namespace pmg
@@ -511,6 +572,18 @@ extern "C" int64_t pmg_mstep_workspace_bytes(int K, int B, int N, int maxiter) {
   (void)K; (void)B; (void)N;
   // barrier word (256-byte header) + partials for up to 1024 CTAs + per-step arrival counters
   return 256 + (int64_t)(maxiter + 1) * 1024 * 2 * (int64_t)sizeof(double) + (int64_t)(maxiter + 1) * 4 + 256;
+}
+
+extern "C" int pmg_mstep_plan(int K, int B, int N, int maxiter, int* kernel, int* phi_in_smem, int* grid, int* parts) {
+  if (K <= 0 || B <= 0 || N <= 0 || maxiter < 1) return PMG_ERR_BAD_ARG;
+  pmg::MstepPlan pl;
+  const int rc = pmg::mstep_plan(K, B, N, pl);
+  if (rc != PMG_OK) return rc;
+  if (kernel) *kernel = pl.lagged;
+  if (phi_in_smem) *phi_in_smem = pl.phi_in_smem;
+  if (grid) *grid = pl.grid;
+  if (parts) *parts = pl.parts;
+  return PMG_OK;
 }
 
 extern "C" int pmg_mstep_adam(int K, int B, int N, const float* Phi, const float* yw, const float* tw,
@@ -534,6 +607,9 @@ extern "C" int pmg_mstep_adam_ld(int K, int B, int N, const float* Phi, const fl
   if (!Phi || !yw || !tw || !W || !mu || !nu || !count || !loss_hist || !err_hist || !n_iter_out || !final_out)
     return PMG_ERR_BAD_ARG;
   if (!workspace || workspace_bytes < pmg_mstep_workspace_bytes(K, B, N, maxiter)) return PMG_ERR_WORKSPACE;
+  MstepPlan pl;
+  const int rc = mstep_plan(K, B, N, pl);
+  if (rc != PMG_OK) return rc;
   cudaStream_t st = (cudaStream_t)stream;
 
   MstepParams p;
@@ -544,60 +620,23 @@ extern "C" int pmg_mstep_adam_ld(int K, int B, int N, const float* Phi, const fl
   p.n_iter_out = n_iter_out; p.final_out = final_out; p.tuning_out = tuning_out;
   p.barrier = (unsigned*)workspace;
   p.partials = (double*)((char*)workspace + 256);
-  p.Bs = B | 1;
-  p.phi_in_smem = mstep_smem(K, B, true, p.Bs) <= 200 * 1024;
-  const size_t smem = mstep_smem(K, B, p.phi_in_smem, p.Bs);
-  if (smem > 227 * 1024) return PMG_ERR_UNSUPPORTED_SHAPE;
+  p.Bs = pl.Bs;
+  p.phi_in_smem = pl.phi_in_smem;
 
   PMG_CUDA_CHECK(cudaMemsetAsync(workspace, 0, 256, st));
   PMG_CUDA_CHECK(cudaMemsetAsync(loss_hist, 0, sizeof(float) * maxiter, st));
   PMG_CUDA_CHECK(cudaMemsetAsync(err_hist, 0, sizeof(float) * maxiter, st));
-  {
-    // lagged-decision kernel: one tile per CTA, all CTAs resident, tile state + operands in shared memory
-    const char* lag_s = std::getenv("PMG_MSTEP_LAG");      // 0 = the barrier-per-step kernel (cross-check)
-    const int lag_env = lag_s ? std::atoi(lag_s) : 1;
-    const int ntiles_l = (N + MS_NT - 1) / MS_NT;
-    constexpr int LT = 512;         // threads per CTA of the lagged kernel (one round over K <= 512 rows of Phi)
-    int Bs_l = B | 1;
-    bool phi_l = mstep_lag_smem<LT>(K, B, true, Bs_l) <= 200 * 1024;
-    const size_t smem_l = mstep_lag_smem<LT>(K, B, phi_l, Bs_l);
-    int dev_l = 0, sms_l = 0, per_l = 0;
-    PMG_CUDA_CHECK(cudaGetDevice(&dev_l));
-    PMG_CUDA_CHECK(cudaDeviceGetAttribute(&sms_l, cudaDevAttrMultiProcessorCount, dev_l));
-    if (lag_env && smem_l <= 200 * 1024) {
-      // attribute + occupancy query once per shared-memory size (host time of a launch that runs every EM iteration)
-      static size_t cached_smem = 0;
-      static int cached_per = 0, cached_dev = -1;
-      if (cached_smem != smem_l || cached_dev != dev_l) {
-        cached_dev = dev_l;
-        PMG_CUDA_CHECK(cudaFuncSetAttribute(mstep_adam_lag_kernel<LT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_l));
-        PMG_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&cached_per, mstep_adam_lag_kernel<LT>, LT, smem_l));
-        cached_smem = smem_l;
-      }
-      per_l = cached_per;
-      if (per_l >= 1 && ntiles_l <= sms_l * per_l && ntiles_l <= 1024) {
-        p.Bs = Bs_l; p.phi_in_smem = phi_l;
-        unsigned* arrived = (unsigned*)((char*)workspace + 256 + (size_t)(maxiter + 1) * 1024 * 2 * sizeof(double));
-        PMG_CUDA_CHECK(cudaMemsetAsync(arrived, 0, (size_t)(maxiter + 1) * sizeof(unsigned), st));
-        void* args_l[] = {(void*)&p, (void*)&arrived};
-        PMG_CUDA_CHECK(cudaLaunchCooperativeKernel((const void*)mstep_adam_lag_kernel<LT>, dim3(ntiles_l), dim3(LT),
-                                                   args_l, smem_l, st));
-        return PMG_OK;
-      }
-    }
+  if (pl.lagged) {
+    unsigned* arrived = (unsigned*)((char*)workspace + 256 + (size_t)(maxiter + 1) * 1024 * 2 * sizeof(double));
+    PMG_CUDA_CHECK(cudaMemsetAsync(arrived, 0, (size_t)(maxiter + 1) * sizeof(unsigned), st));
+    void* args_l[] = {(void*)&p, (void*)&arrived};
+    PMG_CUDA_CHECK(cudaLaunchCooperativeKernel((const void*)mstep_adam_lag_kernel<MS_LAG_THREADS>, dim3(pl.grid),
+                                               dim3(MS_LAG_THREADS), args_l, pl.smem, st));
+  } else {
+    void* args[] = {(void*)&p};
+    PMG_CUDA_CHECK(cudaLaunchCooperativeKernel((const void*)mstep_adam_kernel, dim3(pl.grid), dim3(MS_THREADS), args,
+                                               pl.smem, st));
   }
-  PMG_CUDA_CHECK(cudaFuncSetAttribute(mstep_adam_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  int dev = 0, sms = 0, per_sm = 0;
-  PMG_CUDA_CHECK(cudaGetDevice(&dev));
-  PMG_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-  PMG_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mstep_adam_kernel, MS_THREADS, smem));
-  if (per_sm < 1) return PMG_ERR_UNSUPPORTED_SHAPE;
-  const int ntiles = (N + MS_NT - 1) / MS_NT;
-  int grid = sms * per_sm;
-  if (grid > ntiles) grid = ntiles;
-  if (grid > 1024) grid = 1024;
-  void* args[] = {(void*)&p};
-  PMG_CUDA_CHECK(cudaLaunchCooperativeKernel((const void*)mstep_adam_kernel, dim3(grid), dim3(MS_THREADS), args, smem, st));
   return PMG_OK;
 }
 

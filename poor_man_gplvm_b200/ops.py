@@ -975,6 +975,19 @@ def mstep_adam(Phi, yw, tw, W, state, prior_std, step_size=0.01, maxiter=1000, t
     return loss_hist, err_hist, n_iter, final, tuning
 
 
+def mstep_plan(K, B, N, maxiter=1000):
+    """The launch mstep_adam makes for these shapes on the current device, as the launch itself decides it
+    (PMG_MSTEP_LAG=0 honoured).  Returns dict(kernel="lagged" | "barrier", phi_in_smem, grid, parts,
+    tiles_per_cta): the lagged kernel runs one tile of 4 neurons per CTA; the barrier kernel loops over tiles."""
+    lib = _lib.load()
+    kernel, phi, grid, parts = C.c_int(), C.c_int(), C.c_int(), C.c_int()
+    check(lib.pmg_mstep_plan(int(K), int(B), int(N), int(maxiter), C.byref(kernel), C.byref(phi), C.byref(grid),
+                             C.byref(parts)), "pmg_mstep_plan")
+    ntiles = (int(N) + 3) // 4
+    return {"kernel": "lagged" if kernel.value else "barrier", "phi_in_smem": bool(phi.value), "grid": grid.value,
+            "parts": parts.value, "tiles_per_cta": -(-ntiles // grid.value)}
+
+
 def tuning_softplus(Phi, W):
     """softplus(Phi @ W) (reference fit_tuning_helper.py:11-25)."""
     lib = _lib.load()
