@@ -151,6 +151,16 @@ typedef struct pmg_scan_plan {
   const int* halo_next_arr; /* optional device int32 [n_chain]: per-chain warm-up lengths of the next pass */
 } pmg_scan_plan;
 
+/* Every function that takes a pmg_scan_plan returns PMG_ERR_BAD_ARG unless
+ *   T > 0, 0 <= core_begin < core_end <= T, chunk_len > 0, halo >= 0, halo_next >= 0, and
+ *   (n_chain - 1) * chunk_len < core_end - core_begin <= n_chain * chunk_len (no chain is empty);
+ * those that also take a pmg_transition, ll and a mode (the forward / backward passes of every family) also unless
+ *   K > 0, 0 <= W <= K - 1 (W = 0 when K = 1), kind is 0 (with taps and inv_z) or 1 (with band_fwd for a forward
+ *   pass, band_bwd for a backward pass), ll != NULL, ldll >= K, mode is 0, 1 (with chain_ids and n_ids > 0) or 2
+ *   (with sel_err).
+ * The passes that take no mode (the lockstep passes) check the transition as mode 0.  Conditions that only one family
+ * has (shape limits, alignment, required outputs) are listed with its functions. */
+
 /* mode 0: all chains, warm-up from the uniform carry (left-most chain exact if left_exact).
  * mode 1: relay — run only chains listed in chain_ids[n_ids] (device int32) starting
  *         from the exact carry alpha[t_begin-1].

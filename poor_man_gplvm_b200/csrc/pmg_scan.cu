@@ -12,51 +12,9 @@
 // part through a group reduction that is fused with the normaliser.
 #include <cuda_fp16.h>
 
-#include "pmg_common.cuh"
+#include "pmg_chain.cuh"
 
 namespace pmg {
-
-struct TransDev {
-  int K, kind, W;
-  const float* taps;
-  const float* inv_z;
-  const float* band_fwd;
-  const float* band_bwd;
-  float M00, M01, M10, M11;
-};
-
-struct ScanCommon {
-  int64_t T, core_begin, core_end, chunk_len;
-  int n_chain, halo, left_exact, right_exact;
-  int halo_next;            // warm-up length of the NEXT pass: where warm_out messages are taken
-  const int* halo_arr;      // optional per-chain warm-up lengths of this pass (overrides halo) ...
-  const int* halo_next_arr; // ... and of the next pass (overrides halo_next for chains of this block)
-  const float* sel_err;     // mode 2: chain s runs iff !(sel_err[s] <= sel_tol)
-  float sel_tol;
-  float scale;
-  TransDev tr;
-  const float* ll;
-  int64_t ldll;
-  int mode;
-  const int* chain_ids;
-  int n_ids;
-};
-
-__device__ __forceinline__ int halo_own(const ScanCommon& c, int s) { return c.halo_arr ? c.halo_arr[s] : c.halo; }
-// warm-up length chain j will use in the next pass (j outside this block: the neighbour rank's boundary chain)
-__device__ __forceinline__ int halo_next_of(const ScanCommon& c, int j) {
-  return (c.halo_next_arr && j >= 0 && j < c.n_chain) ? c.halo_next_arr[j] : c.halo_next;
-}
-// mode 2: true when none of this CTA's chains is selected (the CTA returns before touching shared memory)
-__device__ __forceinline__ bool cta_idle(const ScanCommon& c, int chains_per_cta) {
-  if (c.mode != 2) return false;
-  int any = 0;
-  for (int j = threadIdx.x; j < chains_per_cta; j += blockDim.x) {
-    const int s = blockIdx.x * chains_per_cta + j;
-    if (s < c.n_chain && !(c.sel_err[s] <= c.sel_tol)) any = 1;
-  }
-  return __syncthreads_or(any) == 0;
-}
 
 struct FwdParams {
   ScanCommon c;
@@ -110,52 +68,6 @@ struct Geo {
     return sizeof(float) * ((size_t)CPC * (2 * buf_floats(W) + 2 * WPC * 4) + (REG ? 0 : (W + 1)));
   }
 };
-
-// ---- group reductions ------------------------------------------------------
-template <int WPC, int NV>
-__device__ __forceinline__ void group_sum(float (&v)[NV], float* red, int& red_par, int wig, int lane,
-                                          int bar_id) {
-#pragma unroll
-  for (int i = 0; i < NV; ++i) v[i] = warp_sum(v[i]);
-  if (WPC > 1) {
-    float* r = red + red_par * (WPC * 4);
-    if (lane == 0) {
-#pragma unroll
-      for (int i = 0; i < NV; ++i) r[wig * 4 + i] = v[i];
-    }
-    named_bar_sync(bar_id, 32 * WPC);
-#pragma unroll
-    for (int i = 0; i < NV; ++i) {
-      float s = 0.f;
-#pragma unroll
-      for (int w = 0; w < WPC; ++w) s += r[w * 4 + i];
-      v[i] = s;
-    }
-    red_par ^= 1;
-  }
-}
-
-template <int WPC>
-__device__ __forceinline__ float group_max(float v, float* red, int& red_par, int wig, int lane, int bar_id) {
-  v = warp_max(v);
-  if (WPC > 1) {
-    float* r = red + red_par * (WPC * 4);
-    if (lane == 0) r[wig * 4] = v;
-    named_bar_sync(bar_id, 32 * WPC);
-    float s = r[0];
-#pragma unroll
-    for (int w = 1; w < WPC; ++w) s = fmaxf(s, r[w * 4]);
-    v = s;
-    red_par ^= 1;
-  }
-  return v;
-}
-
-template <int WPC>
-__device__ __forceinline__ void group_sync(int bar_id) {
-  if (WPC > 1) named_bar_sync(bar_id, 32 * WPC);
-  else __syncwarp();
-}
 
 // ---- banded "move" operator ------------------------------------------------
 // in[q]  : this thread's Q entries of the input vector (already scaled for the Toeplitz forward case)
@@ -213,28 +125,6 @@ __device__ __forceinline__ int own_x(int gl, int q) {
   return Geo<Q, WPC, WT>::REG ? gl * Q + q : gl + Geo<Q, WPC, WT>::G * q;
 }
 
-// chain bookkeeping shared by both directions
-struct ChainRange {
-  int s;
-  int64_t t_begin, t_end;
-};
-template <int CPC>
-__device__ __forceinline__ bool chain_range(const ScanCommon& c, int grp, ChainRange& r) {
-  int idx = blockIdx.x * CPC + grp;
-  if (c.mode == 1) {
-    if (idx >= c.n_ids) return false;
-    r.s = c.chain_ids[idx];
-  } else {
-    r.s = idx;
-  }
-  if (r.s < 0 || r.s >= c.n_chain) return false;
-  if (c.mode == 2 && c.sel_err[r.s] <= c.sel_tol) return false;   // device-side selection (NaN selects)
-  r.t_begin = c.core_begin + (int64_t)r.s * c.chunk_len;
-  r.t_end = r.t_begin + c.chunk_len;
-  if (r.t_end > c.core_end) r.t_end = c.core_end;
-  return r.t_begin < r.t_end;
-}
-
 // ============================================================================
 // forward
 // ============================================================================
@@ -289,25 +179,9 @@ __global__ void __launch_bounds__(256, 1) fwd_kernel(const FwdParams p) {
   // ---- initial carry
   int64_t t0;
   float al0[Q], al1[Q];
-  bool from_array = false;
-  const float* src = nullptr;
-  if (c.mode != 0) {
-    t0 = cr.t_begin;
-    if (p.warm_in) { from_array = true; src = p.warm_in + (size_t)cr.s * p.warm_stride; }   // snapshot of the carry
-    else if (t0 > 0) { from_array = true; src = p.alpha + (size_t)(t0 - 1) * 2 * K; }
-    else if (p.carry_in) { from_array = true; src = p.carry_in; }
-  } else {
-    t0 = cr.t_begin - halo_own(c, cr.s);
-    if (t0 <= 0 && c.left_exact) {
-      t0 = 0;
-      if (p.carry_in) { from_array = true; src = p.carry_in; }
-    } else {
-      if (t0 < 0) t0 = 0;
-      if (p.warm_in) { from_array = true; src = p.warm_in + (size_t)cr.s * p.warm_stride; }
-    }
-  }
+  const float* src = fwd_start<true>(c, cr, p, t0, K);
   float p1;
-  if (from_array) {
+  if (src) {
     float s2[2] = {0.f, 0.f};
 #pragma unroll
     for (int q = 0; q < Q; ++q) {
@@ -475,22 +349,7 @@ __global__ void __launch_bounds__(256, 1) bwd_kernel(const BwdParams p) {
 
   // ---- where the recursion starts
   int64_t t_hi;
-  const float* init = nullptr;
-  if (c.mode != 0) {
-    if (cr.t_end < c.T) {
-      t_hi = cr.t_end;
-      init = p.warm_in ? p.warm_in + (size_t)cr.s * p.warm_stride : p.beta_end + (size_t)(cr.s + 1) * 2 * K;
-    } else { t_hi = c.T - 1; init = p.beta_in; }
-  } else {
-    t_hi = cr.t_end - 1 + halo_own(c, cr.s);
-    if (t_hi >= c.T - 1 && c.right_exact) {
-      t_hi = c.T - 1;
-      init = p.beta_in;
-    } else {
-      if (t_hi > c.T - 1) t_hi = c.T - 1;
-      if (p.warm_in) init = p.warm_in + (size_t)cr.s * p.warm_stride;
-    }
-  }
+  const float* init = bwd_start<true>(c, cr, p, t_hi, K);
 
   float be0[Q], be1[Q], Lb[Q], tw_acc[Q];
   float RL = 0.f;
@@ -744,7 +603,6 @@ static int bulk_launch(const P& p, int n_groups, cudaStream_t st) {
   if constexpr (FWD) return launch_fwd_bulk<Q, WT, NW, OB>(p, n_groups, st);
   else return launch_bwd_bulk<Q, WT, NW, OB>(p, n_groups, st);
 }
-// choose (Q, WPC): smallest group that covers K with at most 16 bins per thread
 template <bool FWD, typename P>
 static int dispatch(const P& p, int n_groups, cudaStream_t st) {
   const int K = p.c.tr.K;
@@ -754,61 +612,18 @@ static int dispatch(const P& p, int n_groups, cudaStream_t st) {
   // measured on B200)
   const bool w5 = p.c.tr.W <= 5;
   const bool bulk = reg && (K % 8 == 0) && (p.c.ldll % 4 == 0) && bulk_ok(p) && p.c.scale > 0.f;
-#define PMG_CASE(Qv, WPCv)                                                                     \
-  do {                                                                                         \
-    if (bulk && WPCv == 1) {                                                                   \
-      int rc_;                                                                                 \
-      if (w5) rc_ = bulk_launch<FWD, Qv, 5, 8, 2>(p, n_groups, st);                           \
-      else rc_ = bulk_launch<FWD, Qv, 10, 8, 2>(p, n_groups, st);                              \
-      if (rc_ != PMG_ERR_UNSUPPORTED_SHAPE) return rc_;                                        \
-    }                                                                                          \
-    if (wants_xi16(p)) return PMG_ERR_UNSUPPORTED_SHAPE;   /* only the bulk kernel writes them */ \
-    if (reg) {                                                                                 \
-      if constexpr (FWD) return launch_fwd<Qv, WPCv, kRegWT>(p, n_groups, st);                 \
-      else return launch_bwd<Qv, WPCv, kRegWT>(p, n_groups, st);                               \
-    } else {                                                                                   \
-      if constexpr (FWD) return launch_fwd<Qv, WPCv, 0>(p, n_groups, st);                      \
-      else return launch_bwd<Qv, WPCv, 0>(p, n_groups, st);                                    \
-    }                                                                                          \
-  } while (0)
-  if (K <= 32 * 4) PMG_CASE(4, 1);
-  if (K <= 32 * 8) PMG_CASE(8, 1);
-  if (K <= 32 * 13) PMG_CASE(13, 1);
-  if (K <= 32 * 16) PMG_CASE(16, 1);
-  if (K <= 64 * 16) PMG_CASE(16, 2);
-  if (K <= 128 * 16) PMG_CASE(16, 4);
-  if (K <= 256 * 16) PMG_CASE(16, 8);
-#undef PMG_CASE
-  return PMG_ERR_UNSUPPORTED_SHAPE;
-}
-
-static int fill_common(ScanCommon& c, const pmg_scan_plan* plan, const pmg_transition* tr, const float* ll,
-                       int64_t ldll, int mode, const int* chain_ids, int n_ids) {
-  if (!plan || !tr || !ll) return PMG_ERR_BAD_ARG;
-  if (plan->T <= 0 || plan->core_begin < 0 || plan->core_end > plan->T || plan->core_begin >= plan->core_end)
-    return PMG_ERR_BAD_ARG;
-  if (plan->chunk_len <= 0 || plan->halo < 0) return PMG_ERR_BAD_ARG;
-  if ((int64_t)plan->n_chain * plan->chunk_len < plan->core_end - plan->core_begin) return PMG_ERR_BAD_ARG;
-  if (tr->K <= 0 || tr->W < 0 || tr->W > tr->K - 1 + (tr->K == 1)) return PMG_ERR_BAD_ARG;
-  if (tr->kind == 0 && (!tr->taps || !tr->inv_z)) return PMG_ERR_BAD_ARG;
-  if (tr->kind == 1 && (!tr->band_fwd || !tr->band_bwd)) return PMG_ERR_BAD_ARG;
-  if (tr->kind != 0 && tr->kind != 1) return PMG_ERR_BAD_ARG;
-  if (mode == 1 && (!chain_ids || n_ids <= 0)) return PMG_ERR_BAD_ARG;
-  if (mode == 2 && !plan->sel_err) return PMG_ERR_BAD_ARG;
-  if (mode < 0 || mode > 2 || plan->halo_next < 0) return PMG_ERR_BAD_ARG;
-  if (ldll < tr->K) return PMG_ERR_BAD_ARG;
-  c.T = plan->T; c.core_begin = plan->core_begin; c.core_end = plan->core_end;
-  c.chunk_len = plan->chunk_len; c.n_chain = plan->n_chain; c.halo = plan->halo;
-  c.halo_next = plan->halo_next > 0 ? plan->halo_next : plan->halo;
-  c.sel_err = plan->sel_err; c.sel_tol = plan->sel_tol;
-  c.halo_arr = plan->halo_arr; c.halo_next_arr = plan->halo_next_arr;
-  c.left_exact = plan->left_exact; c.right_exact = plan->right_exact;
-  c.scale = plan->likelihood_scale;
-  c.tr.K = tr->K; c.tr.kind = tr->kind; c.tr.W = tr->W;
-  c.tr.taps = tr->taps; c.tr.inv_z = tr->inv_z; c.tr.band_fwd = tr->band_fwd; c.tr.band_bwd = tr->band_bwd;
-  c.tr.M00 = tr->M[0]; c.tr.M01 = tr->M[1]; c.tr.M10 = tr->M[2]; c.tr.M11 = tr->M[3];
-  c.ll = ll; c.ldll = ldll; c.mode = mode; c.chain_ids = chain_ids; c.n_ids = n_ids;
-  return PMG_OK;
+  return by_tier(K, [&](auto Qc, auto WPCc) -> int {
+    constexpr int Qv = Qc, WPCv = WPCc;
+    if constexpr (WPCv == 1) {
+      if (bulk) {
+        const int rc = w5 ? bulk_launch<FWD, Qv, 5, 8, 2>(p, n_groups, st) : bulk_launch<FWD, Qv, 10, 8, 2>(p, n_groups, st);
+        if (rc != PMG_ERR_UNSUPPORTED_SHAPE) return rc;
+      }
+    }
+    if (wants_xi16(p)) return PMG_ERR_UNSUPPORTED_SHAPE;   // only the bulk kernel writes them
+    if constexpr (FWD) return reg ? launch_fwd<Qv, WPCv, kRegWT>(p, n_groups, st) : launch_fwd<Qv, WPCv, 0>(p, n_groups, st);
+    else return reg ? launch_bwd<Qv, WPCv, kRegWT>(p, n_groups, st) : launch_bwd<Qv, WPCv, 0>(p, n_groups, st);
+  });
 }
 
 }  // namespace pmg
@@ -818,7 +633,7 @@ extern "C" int pmg_forward(const pmg_scan_plan* plan, const pmg_transition* tr, 
                            float* alpha, float* lmr, float* halo_state, int mode,
                            const int* chain_ids, int n_ids, pmg_stream_t stream) {
   pmg::FwdParams p;
-  int rc = pmg::fill_common(p.c, plan, tr, ll, ldll, mode, chain_ids, n_ids);
+  int rc = pmg::fill_common(p.c, plan, tr, ll, ldll, mode, chain_ids, n_ids, true);
   if (rc) return rc;
   if (!alpha || !lmr) return PMG_ERR_BAD_ARG;
   p.carry_in = carry_in; p.warm_in = warm_in; p.warm_stride = warm_stride; p.warm_out = warm_out; p.alpha = alpha; p.lmr = lmr; p.halo_state = halo_state;
@@ -833,8 +648,9 @@ static int backward_impl(const pmg_scan_plan* plan, const pmg_transition* tr, co
                          float* tw_partial, float* beta_halo, float* beta_end, int mode, const int* chain_ids, int n_ids,
                          pmg_stream_t stream) {
   pmg::BwdParams p;
-  int rc = pmg::fill_common(p.c, plan, tr, ll, ldll, mode, chain_ids, n_ids);
+  int rc = pmg::fill_common(p.c, plan, tr, ll, ldll, mode, chain_ids, n_ids, false);
   if (rc) return rc;
+  if (xa_hi && !pmg_backward_xi16_supported(tr, plan->likelihood_scale)) return PMG_ERR_UNSUPPORTED_SHAPE;
   if (!alpha) return PMG_ERR_BAD_ARG;
   if (mode != 0 && !beta_end && !warm_in) return PMG_ERR_BAD_ARG;
   if (gamma16 && (ldg < tr->K || (ldg & 7))) return PMG_ERR_BAD_ARG;
@@ -875,7 +691,6 @@ extern "C" int pmg_backward_xi16(const pmg_scan_plan* plan, const pmg_transition
                                  float* tw_partial, float* beta_halo, float* beta_end, int mode, const int* chain_ids,
                                  int n_ids, pmg_stream_t stream) {
   if (!xa_hi) return PMG_ERR_BAD_ARG;
-  if (!pmg_backward_xi16_supported(tr, plan ? plan->likelihood_scale : 0.f)) return PMG_ERR_UNSUPPORTED_SHAPE;
   return backward_impl(plan, tr, ll, ldll, alpha, beta_in, warm_in, warm_stride, warm_out, gamma, gamma_lat, gamma16, ldg,
                        dyn_marg, nullptr, xa_hi, xa_lo, xr_hi, xr_lo, ld_x, tw_partial, beta_halo, beta_end, mode,
                        chain_ids, n_ids, stream);

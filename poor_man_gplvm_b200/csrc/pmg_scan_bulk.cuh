@@ -87,17 +87,7 @@ __global__ void __launch_bounds__(32 * NW, 1) fwd_bulk_kernel(const FwdParams p,
   __syncthreads();
 
   ChainRange cr;
-  {
-    // chain_range() with a compile-time chains-per-CTA
-    int idx = blockIdx.x * NW + grp;
-    if (c.mode == 1) { if (idx >= c.n_ids) return; cr.s = c.chain_ids[idx]; } else cr.s = idx;
-    if (cr.s < 0 || cr.s >= c.n_chain) return;
-    if (c.mode == 2 && c.sel_err[cr.s] <= c.sel_tol) return;
-    cr.t_begin = c.core_begin + (int64_t)cr.s * c.chunk_len;
-    cr.t_end = cr.t_begin + c.chunk_len;
-    if (cr.t_end > c.core_end) cr.t_end = c.core_end;
-    if (cr.t_begin >= cr.t_end) return;
-  }
+  if (!chain_range<NW>(c, grp, cr)) return;
 
   float tp[2 * WT + 1];
 #pragma unroll
@@ -120,22 +110,7 @@ __global__ void __launch_bounds__(32 * NW, 1) fwd_bulk_kernel(const FwdParams p,
   // ---- initial carry (same rules as fwd_kernel): v = alpha_{t0-1} (normalised), inv_prev = 1
   int64_t t0;
   float v0[Q], v1[Q];
-  const float* src = nullptr;
-  if (c.mode != 0) {
-    t0 = cr.t_begin;
-    if (p.warm_in) src = p.warm_in + (size_t)cr.s * p.warm_stride;     // snapshot of the carry
-    else if (t0 > 0) src = p.alpha + (size_t)(t0 - 1) * 2 * K;
-    else if (p.carry_in) src = p.carry_in;
-  } else {
-    t0 = cr.t_begin - halo_own(c, cr.s);
-    if (t0 <= 0 && c.left_exact) {
-      t0 = 0;
-      if (p.carry_in) src = p.carry_in;
-    } else {
-      if (t0 < 0) t0 = 0;
-      if (p.warm_in) src = p.warm_in + (size_t)cr.s * p.warm_stride;
-    }
-  }
+  const float* src = fwd_start<true>(c, cr, p, t0, K);
   float S0 = 0.f, S1 = 0.f;
 #pragma unroll
   for (int q = 0; q < Q; ++q) {
@@ -308,16 +283,7 @@ __global__ void __launch_bounds__(32 * NW, 1) bwd_bulk_kernel(const BwdParams p,
   __syncthreads();
 
   ChainRange cr;
-  {
-    int idx = blockIdx.x * NW + grp;
-    if (c.mode == 1) { if (idx >= c.n_ids) return; cr.s = c.chain_ids[idx]; } else cr.s = idx;
-    if (cr.s < 0 || cr.s >= c.n_chain) return;
-    if (c.mode == 2 && c.sel_err[cr.s] <= c.sel_tol) return;
-    cr.t_begin = c.core_begin + (int64_t)cr.s * c.chunk_len;
-    cr.t_end = cr.t_begin + c.chunk_len;
-    if (cr.t_end > c.core_end) cr.t_end = c.core_end;
-    if (cr.t_begin >= cr.t_end) return;
-  }
+  if (!chain_range<NW>(c, grp, cr)) return;
 
   float tp[2 * WT + 1];
 #pragma unroll
@@ -338,22 +304,7 @@ __global__ void __launch_bounds__(32 * NW, 1) bwd_bulk_kernel(const BwdParams p,
   const float sc2 = c.scale * kLog2e;
 
   int64_t t_hi;
-  const float* init = nullptr;
-  if (c.mode != 0) {
-    if (cr.t_end < c.T) {
-      t_hi = cr.t_end;
-      init = p.warm_in ? p.warm_in + (size_t)cr.s * p.warm_stride : p.beta_end + (size_t)(cr.s + 1) * 2 * K;
-    } else { t_hi = c.T - 1; init = p.beta_in; }
-  } else {
-    t_hi = cr.t_end - 1 + halo_own(c, cr.s);
-    if (t_hi >= c.T - 1 && c.right_exact) {
-      t_hi = c.T - 1;
-      init = p.beta_in;
-    } else {
-      if (t_hi > c.T - 1) t_hi = c.T - 1;
-      if (p.warm_in) init = p.warm_in + (size_t)cr.s * p.warm_stride;
-    }
-  }
+  const float* init = bwd_start<true>(c, cr, p, t_hi, K);
 
   // carried: unnormalised beta b (of the bin handled last), its normaliser inv_prev, its likelihood
   // factor Lb, and RLu = sum_x Lb*b1 (unnormalised jump-state sum)

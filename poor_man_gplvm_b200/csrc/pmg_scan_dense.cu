@@ -19,7 +19,7 @@
 // repairs of individual chains (modes 1, 2) go through the general kernels.
 #include <cuda_fp16.h>
 
-#include "pmg_common.cuh"
+#include "pmg_chain.cuh"
 #include "pmg_tc.cuh"
 
 namespace pmg {
@@ -206,15 +206,9 @@ dense_step_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_con
 // ---------------------------------------------------------------------------------------------
 // per-chain row operations
 // ---------------------------------------------------------------------------------------------
-struct DenseChains {
-  int64_t T, core_begin, core_end, chunk_len;
-  int n_chain, halo, halo_next, left_exact, right_exact, hmax;
-  const int* halo_arr;
-  const int* halo_next_arr;
-  int K;
-  float M00, M01, M10, M11, scale;
-  const float* ll;
-  int64_t ldll;
+// the chain plan (mode 0) and the lockstep operands
+struct DenseChains : ScanCommon {
+  int hmax;                // warm-up steps of the pass: per-chain warm-ups are capped at hmax
   const float* D;          // GEMM result [S_pad, ldd]
   int64_t ldd;
   __half* U16;             // left-hand operand of the next step: [2][S_pad][Kk] fp16 pieces
@@ -252,11 +246,6 @@ struct DenseBwdParams {
   float* beta_halo;
   float* beta_end;
 };
-
-__device__ __forceinline__ int ds_halo_own(const DenseChains& c, int s) { return c.halo_arr ? c.halo_arr[s] : c.halo; }
-__device__ __forceinline__ int ds_halo_next_of(const DenseChains& c, int j) {
-  return (c.halo_next_arr && j >= 0 && j < c.n_chain) ? c.halo_next_arr[j] : c.halo_next;
-}
 
 // block-wide reductions over DS_UPD_THREADS threads; `slot` selects a private scratch row (no reuse hazard
 // between the reductions of one step)
@@ -303,16 +292,14 @@ __global__ void __launch_bounds__(DS_UPD_THREADS) dense_fwd_update_kernel(const 
   __shared__ float red[48];
   const DenseChains& c = p.c;
   const int s = blockIdx.x;
-  const int K = c.K;
   const int64_t t_begin = c.core_begin + (int64_t)s * c.chunk_len;
   int64_t t_end = t_begin + c.chunk_len;
   if (t_end > c.core_end) t_end = c.core_end;
   if (t_begin >= t_end) return;
-  int64_t t0 = t_begin - ds_halo_own(c, s);
-  bool exact = false;
-  if (t0 <= 0 && c.left_exact) { t0 = 0; exact = true; }
-  else if (t0 < 0) t0 = 0;
-  if (t_begin - t0 > c.hmax) { t0 = t_begin - c.hmax; exact = false; }
+  const ChainRange cr{s, t_begin, t_end};
+  const int K = c.tr.K;
+  int64_t t0;
+  const float* src = fwd_start<false>(c, cr, p, t0, K, c.hmax);
   const int j = step - (c.hmax - (int)(t_begin - t0));
   if (j < -1) return;
   const int64_t t = t0 + j;
@@ -326,7 +313,6 @@ __global__ void __launch_bounds__(DS_UPD_THREADS) dense_fwd_update_kernel(const 
   float S0, S1;
   if (j == -1) {
     // ---- initial carry: exact start (carry_in or uniform) or the warm-start message; normalised to unit sum
-    const float* src = exact ? p.carry_in : (p.warm_in ? p.warm_in + (size_t)s * p.warm_stride : nullptr);
     float s0 = 0.f, s1 = 0.f;
 #pragma unroll
     for (int e = 0; e < EPT; ++e) {
@@ -354,7 +340,7 @@ __global__ void __launch_bounds__(DS_UPD_THREADS) dense_fwd_update_kernel(const 
     const float* drow = c.D + (size_t)s * c.ldd;
     const float* lrow = c.ll + (size_t)t * c.ldll;
     const float uscale = st[2];
-    const float p1 = (c.M01 * st[0] + c.M11 * st[1]) * invK;
+    const float p1 = (c.tr.M01 * st[0] + c.tr.M11 * st[1]) * invK;
     float L[EPT];
     float m = -INFINITY;
 #pragma unroll
@@ -398,7 +384,7 @@ __global__ void __launch_bounds__(DS_UPD_THREADS) dense_fwd_update_kernel(const 
         if (x < K) { o[x] = a0[e]; o[K + x] = a1[e]; }
       }
     }
-    if (p.warm_out && t == t_end - ds_halo_next_of(c, s + 1) - 1 && (s + 1 < c.n_chain || !c.right_exact)) {
+    if (p.warm_out && t == t_end - halo_next_of(c, s + 1) - 1 && (s + 1 < c.n_chain || !c.right_exact)) {
       float* o = p.warm_out + (size_t)(s + 1) * 2 * K;
 #pragma unroll
       for (int e = 0; e < EPT; ++e) {
@@ -410,7 +396,7 @@ __global__ void __launch_bounds__(DS_UPD_THREADS) dense_fwd_update_kernel(const 
   // ---- left-hand operand of the next step: u = M00 alpha0 + M10 alpha1 as two scaled fp16 pieces
   float umax = 0.f;
 #pragma unroll
-  for (int e = 0; e < EPT; ++e) { a0[e] = fmaf(c.M00, a0[e], c.M10 * a1[e]); umax = fmaxf(umax, a0[e]); }
+  for (int e = 0; e < EPT; ++e) { a0[e] = fmaf(c.tr.M00, a0[e], c.tr.M10 * a1[e]); umax = fmaxf(umax, a0[e]); }
   umax = block_max(umax, red, 2);
   float inv_scale;
   const float us = piece_scale(umax, &inv_scale);
@@ -428,16 +414,14 @@ __global__ void __launch_bounds__(DS_UPD_THREADS) dense_bwd_update_kernel(const 
   __shared__ float red[48];
   const DenseChains& c = p.c;
   const int s = blockIdx.x;
-  const int K = c.K;
   const int64_t t_begin = c.core_begin + (int64_t)s * c.chunk_len;
   int64_t t_end = t_begin + c.chunk_len;
   if (t_end > c.core_end) t_end = c.core_end;
   if (t_begin >= t_end) return;
-  int64_t t_hi = t_end - 1 + ds_halo_own(c, s);
-  bool exact = false;
-  if (t_hi >= c.T - 1 && c.right_exact) { t_hi = c.T - 1; exact = true; }
-  else if (t_hi > c.T - 1) t_hi = c.T - 1;
-  if (t_hi - (t_end - 1) > c.hmax) { t_hi = t_end - 1 + c.hmax; exact = false; }
+  const ChainRange cr{s, t_begin, t_end};
+  const int K = c.tr.K;
+  int64_t t_hi;
+  const float* init = bwd_start<false>(c, cr, p, t_hi, K, c.hmax);
   const int j = step - (c.hmax - (int)(t_hi - (t_end - 1)));
   if (j < 0) return;
   const int64_t t = t_hi - j;
@@ -448,7 +432,6 @@ __global__ void __launch_bounds__(DS_UPD_THREADS) dense_bwd_update_kernel(const 
   // ---- unnormalised beta_t
   float b0[EPT], b1[EPT];
   if (j == 0) {
-    const float* init = exact ? p.beta_in : (p.warm_in ? p.warm_in + (size_t)s * p.warm_stride : nullptr);
     float sb = 0.f, dummy = 0.f;
 #pragma unroll
     for (int e = 0; e < EPT; ++e) {
@@ -470,8 +453,8 @@ __global__ void __launch_bounds__(DS_UPD_THREADS) dense_bwd_update_kernel(const 
     for (int e = 0; e < EPT; ++e) {
       const int x = threadIdx.x + e * DS_UPD_THREADS;
       const float w0 = x < K ? drow[x] * rscale : 0.f;
-      b0[e] = x < K ? fmaf(c.M00, w0, c.M01 * w1) : 0.f;
-      b1[e] = x < K ? fmaf(c.M10, w0, c.M11 * w1) : 0.f;
+      b0[e] = x < K ? fmaf(c.tr.M00, w0, c.tr.M01 * w1) : 0.f;
+      b1[e] = x < K ? fmaf(c.tr.M10, w0, c.tr.M11 * w1) : 0.f;
     }
   }
   // ---- likelihood factor, normaliser, posterior
@@ -544,7 +527,7 @@ __global__ void __launch_bounds__(DS_UPD_THREADS) dense_bwd_update_kernel(const 
       if (x < K) { o[x] = b0[e] * inv; o[K + x] = b1[e] * inv; }
     }
   }
-  if (p.warm_out && t == t_begin + ds_halo_next_of(c, s - 1) - 1 && (s >= 1 || !c.left_exact)) {
+  if (p.warm_out && t == t_begin + halo_next_of(c, s - 1) - 1 && (s >= 1 || !c.left_exact)) {
     float* o = p.warm_out + ((int64_t)s - 1) * 2 * K;
 #pragma unroll
     for (int e = 0; e < EPT; ++e) {
@@ -609,23 +592,20 @@ static DenseWorkspace dense_workspace(void* base, int n_chain, const DenseGeo& g
   return w;
 }
 
-static int dense_fill_chains(DenseChains& c, const pmg_scan_plan* plan, const pmg_transition* tr, const float* ll,
-                             int64_t ldll, int halo_max, const DenseGeo& g, const DenseWorkspace& w) {
-  if (!plan || !tr || !ll) return PMG_ERR_BAD_ARG;
-  if (plan->T <= 0 || plan->core_begin < 0 || plan->core_end > plan->T || plan->core_begin >= plan->core_end)
-    return PMG_ERR_BAD_ARG;
-  if (plan->chunk_len <= 0 || plan->halo < 0 || plan->halo_next < 0 || halo_max < 0) return PMG_ERR_BAD_ARG;
-  if ((int64_t)plan->n_chain * plan->chunk_len < plan->core_end - plan->core_begin) return PMG_ERR_BAD_ARG;
-  if (tr->K < 16 || tr->K > 256 * DS_MAX_NT || ldll < tr->K) return PMG_ERR_UNSUPPORTED_SHAPE;
-  c.T = plan->T; c.core_begin = plan->core_begin; c.core_end = plan->core_end; c.chunk_len = plan->chunk_len;
-  c.n_chain = plan->n_chain; c.halo = plan->halo; c.halo_next = plan->halo_next > 0 ? plan->halo_next : plan->halo;
-  c.left_exact = plan->left_exact; c.right_exact = plan->right_exact;
-  c.halo_arr = plan->halo_arr; c.halo_next_arr = plan->halo_next_arr;
+// validates plan, transition and operands of a lockstep pass (mode 0) and fills c; g and w receive the geometry and
+// the workspace layout
+static int dense_fill_chains(DenseChains& c, DenseGeo& g, DenseWorkspace& w, const pmg_scan_plan* plan,
+                             const pmg_transition* tr, const void* P16, int halo_max, const float* ll, int64_t ldll,
+                             void* workspace, int64_t workspace_bytes, bool fwd) {
+  const int rc = fill_common(c, plan, tr, ll, ldll, 0, nullptr, 0, fwd);
+  if (rc) return rc;
+  if (!P16 || !workspace || halo_max < 0) return PMG_ERR_BAD_ARG;
+  if (tr->K < 16 || tr->K > 256 * DS_MAX_NT) return PMG_ERR_UNSUPPORTED_SHAPE;
+  if (((uintptr_t)P16 | (uintptr_t)workspace) & 255) return PMG_ERR_ALIGNMENT;
+  g = dense_geo(tr->K);
+  w = dense_workspace(workspace, plan->n_chain, g);
+  if ((int64_t)w.bytes > workspace_bytes) return PMG_ERR_WORKSPACE;
   c.hmax = plan->halo_arr ? (halo_max > plan->halo ? halo_max : plan->halo) : plan->halo;
-  c.K = tr->K;
-  c.M00 = tr->M[0]; c.M01 = tr->M[1]; c.M10 = tr->M[2]; c.M11 = tr->M[3];
-  c.scale = plan->likelihood_scale;
-  c.ll = ll; c.ldll = ldll;
   c.D = w.D; c.ldd = g.Kn;
   c.U16 = w.U16; c.ldu = g.Kk; c.u_piece = (int64_t)w.S_pad * g.Kk;
   c.state = w.state;
@@ -721,15 +701,12 @@ extern "C" int pmg_forward_dense(const pmg_scan_plan* plan, const pmg_transition
                                  float* alpha, float* lmr, float* halo_state, void* workspace,
                                  int64_t workspace_bytes, pmg_stream_t stream) {
   using namespace pmg;
-  if (!plan || !tr || !P16 || !alpha || !lmr || !workspace) return PMG_ERR_BAD_ARG;
-  if (tr->K < 16 || tr->K > 256 * DS_MAX_NT) return PMG_ERR_UNSUPPORTED_SHAPE;
-  if (((uintptr_t)P16 | (uintptr_t)workspace) & 255) return PMG_ERR_ALIGNMENT;
-  const DenseGeo g = dense_geo(tr->K);
-  const DenseWorkspace w = dense_workspace(workspace, plan->n_chain, g);
-  if ((int64_t)w.bytes > workspace_bytes) return PMG_ERR_WORKSPACE;
   DenseFwdParams p;
-  int rc = dense_fill_chains(p.c, plan, tr, ll, ldll, halo_max, g, w);
+  DenseGeo g;
+  DenseWorkspace w;
+  int rc = dense_fill_chains(p.c, g, w, plan, tr, P16, halo_max, ll, ldll, workspace, workspace_bytes, true);
   if (rc) return rc;
+  if (!alpha || !lmr) return PMG_ERR_BAD_ARG;
   p.carry_in = carry_in; p.warm_in = warm_in; p.warm_stride = warm_stride; p.warm_out = warm_out;
   p.alpha = alpha; p.lmr = lmr; p.halo_state = halo_state;
   DenseGemmLaunch L;
@@ -756,16 +733,13 @@ extern "C" int pmg_backward_dense(const pmg_scan_plan* plan, const pmg_transitio
                                   float* beta_halo, float* beta_end, void* workspace, int64_t workspace_bytes,
                                   pmg_stream_t stream) {
   using namespace pmg;
-  if (!plan || !tr || !P16 || !alpha || !workspace) return PMG_ERR_BAD_ARG;
-  if (tr->K < 16 || tr->K > 256 * DS_MAX_NT) return PMG_ERR_UNSUPPORTED_SHAPE;
-  if (gamma16 && (ldg < tr->K || (ldg & 7))) return PMG_ERR_BAD_ARG;
-  if (((uintptr_t)P16 | (uintptr_t)workspace) & 255) return PMG_ERR_ALIGNMENT;
-  const DenseGeo g = dense_geo(tr->K);
-  const DenseWorkspace w = dense_workspace(workspace, plan->n_chain, g);
-  if ((int64_t)w.bytes > workspace_bytes) return PMG_ERR_WORKSPACE;
   DenseBwdParams p;
-  int rc = dense_fill_chains(p.c, plan, tr, ll, ldll, halo_max, g, w);
+  DenseGeo g;
+  DenseWorkspace w;
+  int rc = dense_fill_chains(p.c, g, w, plan, tr, P16, halo_max, ll, ldll, workspace, workspace_bytes, false);
   if (rc) return rc;
+  if (!alpha) return PMG_ERR_BAD_ARG;
+  if (gamma16 && (ldg < tr->K || (ldg & 7))) return PMG_ERR_BAD_ARG;
   p.alpha = alpha; p.beta_in = beta_in; p.warm_in = warm_in; p.warm_stride = warm_stride; p.warm_out = warm_out;
   p.gamma = gamma; p.gamma_lat = gamma_lat; p.gamma16 = (__half*)gamma16; p.ldg = ldg;
   p.dyn_marg = dyn_marg; p.r_out = r_out; p.r_scratch = w.r_scratch; p.tw_partial = tw_partial;

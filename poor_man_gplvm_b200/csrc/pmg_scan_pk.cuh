@@ -232,16 +232,7 @@ __global__ void __launch_bounds__(32 * NW, 1) fwd_c_kernel(const FwdCParams p, c
   __syncthreads();
 
   ChainRange cr;
-  {
-    const int idx = blockIdx.x * NW + grp;
-    if (c.mode == 1) { if (idx >= c.n_ids) return; cr.s = c.chain_ids[idx]; } else cr.s = idx;
-    if (cr.s < 0 || cr.s >= c.n_chain) return;
-    if (c.mode == 2 && c.sel_err[cr.s] <= c.sel_tol) return;
-    cr.t_begin = c.core_begin + (int64_t)cr.s * c.chunk_len;
-    cr.t_end = cr.t_begin + c.chunk_len;
-    if (cr.t_end > c.core_end) cr.t_end = c.core_end;
-    if (cr.t_begin >= cr.t_end) return;
-  }
+  if (!chain_range<NW>(c, grp, cr)) return;
 
   // taps carry M00: prior move message = M00 * band(iz * u), u = v0 + (M10/M00) v1, v1 = p1 * Lc
   const float M00 = c.tr.M00, M01 = c.tr.M01, M11 = c.tr.M11;
@@ -263,21 +254,7 @@ __global__ void __launch_bounds__(32 * NW, 1) fwd_c_kernel(const FwdCParams p, c
 
   // ---- initial carry
   int64_t t0;
-  const float* src = nullptr;
-  if (c.mode != 0) {
-    t0 = cr.t_begin;
-    if (p.warm_in) src = p.warm_in + (size_t)cr.s * p.warm_stride;
-    else if (t0 == 0 && p.carry_in) src = p.carry_in;
-  } else {
-    t0 = cr.t_begin - halo_own(c, cr.s);
-    if (t0 <= 0 && c.left_exact) {
-      t0 = 0;
-      if (p.carry_in) src = p.carry_in;
-    } else {
-      if (t0 < 0) t0 = 0;
-      if (p.warm_in) src = p.warm_in + (size_t)cr.s * p.warm_stride;
-    }
-  }
+  const float* src = fwd_start<false>(c, cr, p, t0, K);   // no alpha to restart from
   // u = v0 + cM * v1 (unnormalised), S0 = sum v0, S1 = sum v1, inv_prev = 1 / (S0 + S1)
   float2 u[QP];
   float S0 = 0.f, S1 = 0.f;
@@ -448,16 +425,7 @@ __global__ void __launch_bounds__(32 * NW, 1) bwd_c_kernel(const BwdCParams p, c
   __syncthreads();
 
   ChainRange cr;
-  {
-    const int idx = blockIdx.x * NW + grp;
-    if (c.mode == 1) { if (idx >= c.n_ids) return; cr.s = c.chain_ids[idx]; } else cr.s = idx;
-    if (cr.s < 0 || cr.s >= c.n_chain) return;
-    if (c.mode == 2 && c.sel_err[cr.s] <= c.sel_tol) return;
-    cr.t_begin = c.core_begin + (int64_t)cr.s * c.chunk_len;
-    cr.t_end = cr.t_begin + c.chunk_len;
-    if (cr.t_end > c.core_end) cr.t_end = c.core_end;
-    if (cr.t_begin >= cr.t_end) return;
-  }
+  if (!chain_range<NW>(c, grp, cr)) return;
 
   float tp[2 * WT + 1];
 #pragma unroll
@@ -478,22 +446,7 @@ __global__ void __launch_bounds__(32 * NW, 1) bwd_c_kernel(const BwdCParams p, c
   const float sc2 = c.scale * kLog2e;
 
   int64_t t_hi;
-  const float* init = nullptr;
-  if (c.mode != 0) {
-    if (cr.t_end < c.T) {
-      t_hi = cr.t_end;
-      init = p.warm_in ? p.warm_in + (size_t)cr.s * p.warm_stride : p.beta_end + (size_t)(cr.s + 1) * 2 * K;
-    } else { t_hi = c.T - 1; init = p.beta_in; }
-  } else {
-    t_hi = cr.t_end - 1 + halo_own(c, cr.s);
-    if (t_hi >= c.T - 1 && c.right_exact) {
-      t_hi = c.T - 1;
-      init = p.beta_in;
-    } else {
-      if (t_hi > c.T - 1) t_hi = c.T - 1;
-      if (p.warm_in) init = p.warm_in + (size_t)cr.s * p.warm_stride;
-    }
-  }
+  const float* init = bwd_start<true>(c, cr, p, t_hi, K);
 
   // carried: unnormalised beta (b0, b1) of the bin handled last, its likelihood factor with the normaliser
   // folded in (Lb), the unnormalised jump-state sum RLu = sum_x E*b1 and the normaliser inv_prev
@@ -758,7 +711,7 @@ extern "C" int pmg_forward_compact(const pmg_scan_plan* plan, const pmg_transiti
                                    float* ax, int64_t ldax, float* halo_state, float* fwd_end, float* first_out,
                                    int mode, const int* chain_ids, int n_ids, pmg_stream_t stream) {
   pmg::FwdCParams p;
-  int rc = pmg::fill_common(p.c, plan, tr, ll, ldll, mode, chain_ids, n_ids);
+  int rc = pmg::fill_common(p.c, plan, tr, ll, ldll, mode, chain_ids, n_ids, true);
   if (rc) return rc;
   if (!ax || ldax < tr->K + 4 || (ldax & 3) || (ldll & 3)) return PMG_ERR_BAD_ARG;
   if (!pmg_scan_compact_supported(tr, plan->likelihood_scale)) return PMG_ERR_UNSUPPORTED_SHAPE;
@@ -776,7 +729,7 @@ extern "C" int pmg_backward_compact(const pmg_scan_plan* plan, const pmg_transit
                                     float* beta_halo, float* beta_end, int mode,
                                     const int* chain_ids, int n_ids, pmg_stream_t stream) {
   pmg::BwdCParams p;
-  int rc = pmg::fill_common(p.c, plan, tr, ll, ldll, mode, chain_ids, n_ids);
+  int rc = pmg::fill_common(p.c, plan, tr, ll, ldll, mode, chain_ids, n_ids, false);
   if (rc) return rc;
   if (!ax || ldax < tr->K + 4 || (ldax & 3) || (ldll & 3)) return PMG_ERR_BAD_ARG;
   if (!gamma16 || ldg < tr->K || (ldg & 7)) return PMG_ERR_BAD_ARG;

@@ -16,26 +16,13 @@
 // backtracks its own chains as pmg_viterbi_backtrack does.
 #include <climits>
 
-#include "pmg_common.cuh"
+#include "pmg_chain.cuh"
 
 namespace pmg {
 namespace vit {
 
 struct Params {
-  int64_t T, core_begin, core_end, chunk_len;
-  int n_chain, halo, halo_next, left_exact, right_exact;
-  const int* halo_arr;
-  const int* halo_next_arr;
-  const float* sel_err;
-  float sel_tol;
-  float scale;
-  int K, kind, W;
-  const float* taps;
-  const float* inv_z;
-  const float* band_fwd;
-  float M00, M01, M10, M11;
-  const float* ll;
-  int64_t ldll;
+  ScanCommon c;
   const float* carry_in;
   const float* warm_in;
   int64_t warm_stride;
@@ -45,9 +32,6 @@ struct Params {
   float* lmr;
   float* halo_state;
   float* end_msg;
-  int mode;
-  const int* chain_ids;
-  int n_ids;
 };
 
 // (value, flat index) order of the max-product: larger value first, then the smaller index
@@ -83,44 +67,6 @@ __device__ __forceinline__ void group_argmax(float& v, int& i, float* red, int& 
   }
 }
 
-template <int WPC>
-__device__ __forceinline__ void group_sum2(float (&v)[2], float* red, int& red_par, int wig, int lane, int bar_id) {
-  v[0] = warp_sum(v[0]);
-  v[1] = warp_sum(v[1]);
-  if (WPC > 1) {
-    float* r = red + red_par * (WPC * 4);
-    if (lane == 0) { r[wig * 4] = v[0]; r[wig * 4 + 1] = v[1]; }
-    named_bar_sync(bar_id, 32 * WPC);
-    float s0 = 0.f, s1 = 0.f;
-#pragma unroll
-    for (int w = 0; w < WPC; ++w) { s0 += r[w * 4]; s1 += r[w * 4 + 1]; }
-    v[0] = s0; v[1] = s1;
-    red_par ^= 1;
-  }
-}
-
-template <int WPC>
-__device__ __forceinline__ float group_max(float v, float* red, int& red_par, int wig, int lane, int bar_id) {
-  v = warp_max(v);
-  if (WPC > 1) {
-    float* r = red + red_par * (WPC * 4);
-    if (lane == 0) r[wig * 4] = v;
-    named_bar_sync(bar_id, 32 * WPC);
-    float s = r[0];
-#pragma unroll
-    for (int w = 1; w < WPC; ++w) s = fmaxf(s, r[w * 4]);
-    v = s;
-    red_par ^= 1;
-  }
-  return v;
-}
-
-template <int WPC>
-__device__ __forceinline__ void group_sync(int bar_id) {
-  if (WPC > 1) named_bar_sync(bar_id, 32 * WPC);
-  else __syncwarp();
-}
-
 __device__ __forceinline__ int16_t as_state(int i, int K2) { return (int16_t)((unsigned)i < (unsigned)K2 ? i : 0); }
 
 template <int Q, int WPC>
@@ -138,15 +84,9 @@ template <int Q, int WPC>
 __global__ void __launch_bounds__(256, 1) viterbi_fwd_kernel(const Params p) {
   using Ge = Geo<Q, WPC>;
   extern __shared__ float smem[];
-  if (p.mode == 2) {   // no chain of this CTA selected: return before touching shared memory
-    int any = 0;
-    for (int j = threadIdx.x; j < Ge::CPC; j += blockDim.x) {
-      const int s = blockIdx.x * Ge::CPC + j;
-      if (s < p.n_chain && !(p.sel_err[s] <= p.sel_tol)) any = 1;
-    }
-    if (__syncthreads_or(any) == 0) return;
-  }
-  const int K = p.K, W = p.W, kind = p.kind, K2 = 2 * K;
+  const ScanCommon& c = p.c;
+  if (cta_idle(c, Ge::CPC)) return;
+  const int K = c.tr.K, W = c.tr.W, kind = c.tr.kind, K2 = 2 * K;
   const int grp = threadIdx.x / Ge::G;
   const int gl = threadIdx.x % Ge::G;
   const int lane = threadIdx.x & 31;
@@ -158,7 +98,7 @@ __global__ void __launch_bounds__(256, 1) viterbi_fwd_kernel(const Params p) {
   float* red = vbuf + 4 * bf;
   float* tapsS = smem + (size_t)Ge::CPC * pc;
   if (kind == 0)
-    for (int i = threadIdx.x; i <= W; i += blockDim.x) tapsS[i] = p.taps[i];
+    for (int i = threadIdx.x; i <= W; i += blockDim.x) tapsS[i] = c.tr.taps[i];
   for (int i = threadIdx.x; i < Ge::CPC * pc; i += blockDim.x) {
     const int o = i % pc;
     if (o < 2 * bf) smem[i] = -1.f;
@@ -167,23 +107,10 @@ __global__ void __launch_bounds__(256, 1) viterbi_fwd_kernel(const Params p) {
   }
   __syncthreads();
 
-  // ---- chain of this group (mode 1: listed chains; mode 2: selected on the device)
-  int s;
-  {
-    const int idx = blockIdx.x * Ge::CPC + grp;
-    if (p.mode == 1) {
-      if (idx >= p.n_ids) return;
-      s = p.chain_ids[idx];
-    } else {
-      s = idx;
-    }
-    if (s < 0 || s >= p.n_chain) return;
-    if (p.mode == 2 && p.sel_err[s] <= p.sel_tol) return;
-  }
-  const int64_t t_begin = p.core_begin + (int64_t)s * p.chunk_len;
-  int64_t t_end = t_begin + p.chunk_len;
-  if (t_end > p.core_end) t_end = p.core_end;
-  if (t_begin >= t_end) return;
+  ChainRange cr;
+  if (!chain_range<Ge::CPC>(c, grp, cr)) return;
+  const int s = cr.s;
+  const int64_t t_begin = cr.t_begin, t_end = cr.t_end;
 
   float invz[Q];
   bool valid[Q];
@@ -191,30 +118,17 @@ __global__ void __launch_bounds__(256, 1) viterbi_fwd_kernel(const Params p) {
   for (int q = 0; q < Q; ++q) {
     const int x = gl + Ge::G * q;
     valid[q] = x < K;
-    invz[q] = (kind == 0 && valid[q]) ? __ldg(p.inv_z + x) : 1.f;
+    invz[q] = (kind == 0 && valid[q]) ? __ldg(c.tr.inv_z + x) : 1.f;
   }
-  const float M00 = p.M00, M01 = p.M01, M10 = p.M10, M11 = p.M11;
+  const float M00 = c.tr.M00, M01 = c.tr.M01, M10 = c.tr.M10, M11 = c.tr.M11;
   const float invK = 1.f / (float)K;
-  const float scale = p.scale;
+  const float scale = c.scale;
   int red_par = 0;
 
   // ---- initial message: the carry in front of bin 0, or a warm start (pmg_forward's conventions)
   int64_t t0;
-  const float* src = nullptr;
-  if (p.mode != 0) {
-    t0 = t_begin;
-    src = t0 > 0 ? p.warm_in + (size_t)s * p.warm_stride : p.carry_in;
-  } else {
-    const int h = p.halo_arr ? p.halo_arr[s] : p.halo;
-    t0 = t_begin - h;
-    if (t0 <= 0 && p.left_exact) {
-      t0 = 0;
-      src = p.carry_in;
-    } else {
-      if (t0 < 0) t0 = 0;
-      if (p.warm_in) src = p.warm_in + (size_t)s * p.warm_stride;
-    }
-  }
+  const float* src = fwd_start<false>(c, cr, p, t0, K);
+  if (c.mode != 0 && t0 == 0) src = p.carry_in;   // a restart at bin 0 starts from the carry, not the snapshot
   float de0[Q], de1[Q];   // the normalised message delta-hat (move, jump)
   float p1 = 0.f;         // jump-state prior of a sum-product step (bin 0)
   {
@@ -229,7 +143,7 @@ __global__ void __launch_bounds__(256, 1) viterbi_fwd_kernel(const Params p) {
         s2[0] += de0[q];
         s2[1] += de1[q];
       }
-      group_sum2<WPC>(s2, red, red_par, wig, lane, bar_id);
+      group_sum<WPC, 2>(s2, red, red_par, wig, lane, bar_id);
       const float tot = s2[0] + s2[1];
       if (tot > 0.f && tot < 3.0e38f) {
         const float inv = 1.f / tot;
@@ -249,7 +163,7 @@ __global__ void __launch_bounds__(256, 1) viterbi_fwd_kernel(const Params p) {
 
   float lln[Q];
   {
-    const float* row = p.ll + (size_t)t0 * p.ldll;
+    const float* row = c.ll + (size_t)t0 * c.ldll;
 #pragma unroll
     for (int q = 0; q < Q; ++q) lln[q] = valid[q] ? __ldg(row + gl + Ge::G * q) : -INFINITY;
   }
@@ -260,7 +174,7 @@ __global__ void __launch_bounds__(256, 1) viterbi_fwd_kernel(const Params p) {
 #pragma unroll
     for (int q = 0; q < Q; ++q) llc[q] = lln[q];
     if (t + 1 < t_end) {
-      const float* row = p.ll + (size_t)(t + 1) * p.ldll;
+      const float* row = c.ll + (size_t)(t + 1) * c.ldll;
 #pragma unroll
       for (int q = 0; q < Q; ++q) lln[q] = valid[q] ? __ldg(row + gl + Ge::G * q) : -INFINITY;
     }
@@ -291,7 +205,7 @@ __global__ void __launch_bounds__(256, 1) viterbi_fwd_kernel(const Params p) {
           for (int j = 0; j <= 2 * W; ++j) {
             const int x = x1 - W + j;
             if ((unsigned)x >= (unsigned)K) continue;
-            const float w = kind == 0 ? tapsS[j >= W ? j - W : W - j] : __ldg(p.band_fwd + (size_t)j * K + x1);
+            const float w = kind == 0 ? tapsS[j >= W ? j - W : W - j] : __ldg(c.tr.band_fwd + (size_t)j * K + x1);
             acc = fmaf(w, vb[x1 + j], acc);
           }
         }
@@ -327,15 +241,15 @@ __global__ void __launch_bounds__(256, 1) viterbi_fwd_kernel(const Params p) {
         if (valid[q]) {
           if (kind == 0) {
             for (int j = 0; j <= 2 * W; ++j) {
-              const float c = tapsS[j >= W ? j - W : W - j] * vb[x1 + j];
+              const float cv = tapsS[j >= W ? j - W : W - j] * vb[x1 + j];
               const int ci = ib[x1 + j];
-              if (better(c, ci, bv, bi)) { bv = c; bi = ci; }
+              if (better(cv, ci, bv, bi)) { bv = cv; bi = ci; }
             }
           } else {
             for (int j = 0; j <= 2 * W; ++j) {
-              const float c = __ldg(p.band_fwd + (size_t)j * K + x1) * vb[x1 + j];
+              const float cv = __ldg(c.tr.band_fwd + (size_t)j * K + x1) * vb[x1 + j];
               const int ci = ib[x1 + j];
-              if (better(c, ci, bv, bi)) { bv = c; bi = ci; }
+              if (better(cv, ci, bv, bi)) { bv = cv; bi = ci; }
             }
           }
         }
@@ -353,7 +267,7 @@ __global__ void __launch_bounds__(256, 1) viterbi_fwd_kernel(const Params p) {
       s2[0] += de0[q];
       s2[1] += de1[q];
     }
-    group_sum2<WPC>(s2, red, red_par, wig, lane, bar_id);
+    group_sum<WPC, 2>(s2, red, red_par, wig, lane, bar_id);
     const float cn = s2[0] + s2[1];
     const float inv = 1.f / cn;
 #pragma unroll
@@ -384,8 +298,7 @@ __global__ void __launch_bounds__(256, 1) viterbi_fwd_kernel(const Params p) {
     }
     if (p.warm_out) {
       const int j = s + 1;
-      const int hn = (p.halo_next_arr && j < p.n_chain) ? p.halo_next_arr[j] : p.halo_next;
-      if (t == t_end - hn - 1 && (j < p.n_chain || !p.right_exact)) {
+      if (t == t_end - halo_next_of(c, j) - 1 && (j < c.n_chain || !c.right_exact)) {
         float* o = p.warm_out + (size_t)j * K2;
 #pragma unroll
         for (int q = 0; q < Q; ++q)
@@ -507,33 +420,13 @@ __global__ void __launch_bounds__(128) viterbi_fill_kernel(int K, int n_chain, i
 template <int Q, int WPC>
 static int launch(const Params& p, int n_groups, cudaStream_t st) {
   using Ge = Geo<Q, WPC>;
-  const size_t smem = Ge::smem_bytes(p.W);
+  const size_t smem = Ge::smem_bytes(p.c.tr.W);
   if (smem > 227 * 1024) return PMG_ERR_UNSUPPORTED_SHAPE;
   PMG_CUDA_CHECK(cudaFuncSetAttribute(viterbi_fwd_kernel<Q, WPC>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                       (int)smem));
   viterbi_fwd_kernel<Q, WPC><<<cdiv(n_groups, Ge::CPC), 256, smem, st>>>(p);
   PMG_LAUNCH_CHECK();
   return PMG_OK;
-}
-
-// smallest group that covers K with at most 16 bins per thread (pmg_forward's table)
-static int dispatch(const Params& p, int n_groups, cudaStream_t st) {
-  const int K = p.K;
-  if (K <= 32 * 4) return launch<4, 1>(p, n_groups, st);
-  if (K <= 32 * 8) return launch<8, 1>(p, n_groups, st);
-  if (K <= 32 * 13) return launch<13, 1>(p, n_groups, st);
-  if (K <= 32 * 16) return launch<16, 1>(p, n_groups, st);
-  if (K <= 64 * 16) return launch<16, 2>(p, n_groups, st);
-  if (K <= 128 * 16) return launch<16, 4>(p, n_groups, st);
-  if (K <= 256 * 16) return launch<16, 8>(p, n_groups, st);
-  return PMG_ERR_UNSUPPORTED_SHAPE;
-}
-
-static bool plan_ok(const pmg_scan_plan* plan) {
-  return plan && plan->T > 0 && plan->core_begin >= 0 && plan->core_end <= plan->T &&
-         plan->core_begin < plan->core_end && plan->chunk_len > 0 && plan->halo >= 0 && plan->n_chain > 0 &&
-         (int64_t)plan->n_chain * plan->chunk_len >= plan->core_end - plan->core_begin &&
-         (int64_t)(plan->n_chain - 1) * plan->chunk_len < plan->core_end - plan->core_begin;
 }
 
 }  // namespace vit
@@ -543,34 +436,21 @@ extern "C" int pmg_viterbi_forward(const pmg_scan_plan* plan, const pmg_transiti
                                    int64_t ldll, const float* carry_in, const float* warm_in, int64_t warm_stride,
                                    float* warm_out, void* bp, int64_t ldbp, float* lmr, float* halo_state,
                                    float* end_msg, int mode, const int* chain_ids, int n_ids, pmg_stream_t stream) {
-  using namespace pmg::vit;
-  if (!pmg::vit::plan_ok(plan) || !tr || !ll || !bp || !lmr) return PMG_ERR_BAD_ARG;
-  if (tr->K <= 0 || tr->K > 4096 || tr->W < 0 || tr->W > tr->K - 1 + (tr->K == 1)) return PMG_ERR_BAD_ARG;
-  if (tr->kind == 0 && (!tr->taps || !tr->inv_z)) return PMG_ERR_BAD_ARG;
-  if (tr->kind == 1 && !tr->band_fwd) return PMG_ERR_BAD_ARG;
-  if (tr->kind != 0 && tr->kind != 1) return PMG_ERR_BAD_ARG;
-  if (mode < 0 || mode > 2 || plan->halo_next < 0) return PMG_ERR_BAD_ARG;
-  if (mode == 1 && (!chain_ids || n_ids <= 0)) return PMG_ERR_BAD_ARG;
-  if (mode == 2 && !plan->sel_err) return PMG_ERR_BAD_ARG;
+  pmg::vit::Params p;
+  const int rc = pmg::fill_common(p.c, plan, tr, ll, ldll, mode, chain_ids, n_ids, true);
+  if (rc) return rc;
+  if (!bp || !lmr || tr->K > 4096 || ldbp < tr->K) return PMG_ERR_BAD_ARG;
   if (mode != 0 && !warm_in) return PMG_ERR_BAD_ARG;   // restarts begin from a snapshot of the carry
-  if (ldll < tr->K || ldbp < tr->K) return PMG_ERR_BAD_ARG;
-  Params p;
-  p.T = plan->T; p.core_begin = plan->core_begin; p.core_end = plan->core_end; p.chunk_len = plan->chunk_len;
-  p.n_chain = plan->n_chain; p.halo = plan->halo; p.halo_next = plan->halo_next > 0 ? plan->halo_next : plan->halo;
-  p.left_exact = plan->left_exact; p.right_exact = plan->right_exact;
-  p.halo_arr = plan->halo_arr; p.halo_next_arr = plan->halo_next_arr;
-  p.sel_err = plan->sel_err; p.sel_tol = plan->sel_tol; p.scale = plan->likelihood_scale;
-  p.K = tr->K; p.kind = tr->kind; p.W = tr->W; p.taps = tr->taps; p.inv_z = tr->inv_z; p.band_fwd = tr->band_fwd;
-  p.M00 = tr->M[0]; p.M01 = tr->M[1]; p.M10 = tr->M[2]; p.M11 = tr->M[3];
-  p.ll = ll; p.ldll = ldll; p.carry_in = carry_in; p.warm_in = warm_in; p.warm_stride = warm_stride;
-  p.warm_out = warm_out; p.bp = (int16_t*)bp; p.ldbp = ldbp; p.lmr = lmr; p.halo_state = halo_state;
-  p.end_msg = end_msg; p.mode = mode; p.chain_ids = chain_ids; p.n_ids = n_ids;
-  return dispatch(p, mode == 1 ? n_ids : plan->n_chain, (cudaStream_t)stream);
+  p.carry_in = carry_in; p.warm_in = warm_in; p.warm_stride = warm_stride; p.warm_out = warm_out;
+  p.bp = (int16_t*)bp; p.ldbp = ldbp; p.lmr = lmr; p.halo_state = halo_state; p.end_msg = end_msg;
+  return pmg::by_tier(tr->K, [&](auto Q, auto WPC) {
+    return pmg::vit::launch<Q, WPC>(p, mode == 1 ? n_ids : plan->n_chain, (cudaStream_t)stream);
+  });
 }
 
 extern "C" int pmg_viterbi_chain_maps(const pmg_scan_plan* plan, int K, const void* bp, int64_t ldbp, int* maps,
                                       pmg_stream_t stream) {
-  if (!pmg::vit::plan_ok(plan) || !bp || !maps || K <= 0 || K > 4096 || ldbp < K) return PMG_ERR_BAD_ARG;
+  if (!pmg::plan_ok(plan) || !bp || !maps || K <= 0 || K > 4096 || ldbp < K) return PMG_ERR_BAD_ARG;
   const dim3 grid(plan->n_chain, pmg::cdiv(2 * K, 256));
   pmg::vit::viterbi_maps_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(K, plan->core_begin, plan->core_end,
                                                                        plan->chunk_len, (const int16_t*)bp, ldbp,
@@ -581,7 +461,7 @@ extern "C" int pmg_viterbi_chain_maps(const pmg_scan_plan* plan, int K, const vo
 
 extern "C" int pmg_viterbi_backtrack(const pmg_scan_plan* plan, int K, const void* bp, int64_t ldbp,
                                      const int* maps, const float* last_msg, int* path, pmg_stream_t stream) {
-  if (!pmg::vit::plan_ok(plan) || !bp || !maps || !last_msg || !path || K <= 0 || K > 4096 || ldbp < K)
+  if (!pmg::plan_ok(plan) || !bp || !maps || !last_msg || !path || K <= 0 || K > 4096 || ldbp < K)
     return PMG_ERR_BAD_ARG;
   cudaStream_t st = (cudaStream_t)stream;
   pmg::vit::viterbi_resolve_kernel<<<1, 256, 0, st>>>(K, plan->n_chain, plan->core_begin, plan->core_end,
@@ -596,7 +476,7 @@ extern "C" int pmg_viterbi_backtrack(const pmg_scan_plan* plan, int K, const voi
 
 extern "C" int pmg_viterbi_block_link(const pmg_scan_plan* plan, int K, const void* bp, int64_t ldbp, const int* maps,
                                       int* link, pmg_stream_t stream) {
-  if (!pmg::vit::plan_ok(plan) || plan->core_begin < 1 || !bp || !maps || !link || K <= 0 || K > 4096 || ldbp < K)
+  if (!pmg::plan_ok(plan) || plan->core_begin < 1 || !bp || !maps || !link || K <= 0 || K > 4096 || ldbp < K)
     return PMG_ERR_BAD_ARG;
   pmg::vit::viterbi_link_kernel<<<pmg::cdiv(2 * K, 256), 256, 0, (cudaStream_t)stream>>>(
       K, plan->n_chain, plan->core_begin, plan->core_end, plan->chunk_len, (const int16_t*)bp, ldbp, maps, link);
@@ -607,7 +487,7 @@ extern "C" int pmg_viterbi_block_link(const pmg_scan_plan* plan, int K, const vo
 extern "C" int pmg_viterbi_backtrack_sharded(const pmg_scan_plan* plan, int K, const void* bp, int64_t ldbp,
                                              const int* maps, const int* gathered, int world, int rank, int* path,
                                              pmg_stream_t stream) {
-  if (!pmg::vit::plan_ok(plan) || !bp || !maps || !gathered || !path || K <= 0 || K > 4096 || ldbp < K ||
+  if (!pmg::plan_ok(plan) || !bp || !maps || !gathered || !path || K <= 0 || K > 4096 || ldbp < K ||
       world < 1 || rank < 0 || rank >= world)
     return PMG_ERR_BAD_ARG;
   cudaStream_t st = (cudaStream_t)stream;

@@ -534,31 +534,27 @@ def set_chain_halos(plan, cur=None, nxt=None):
     plan.halo_next_arr = nxt.data_ptr() if nxt is not None else None
 
 
-def _select(plan, mode, sel_err, sel_tol):
-    """mode 2: the chains to re-run are selected on the device, chain s iff !(sel_err[s] <= sel_tol)."""
+def _pass_args(plan, op, mode, chain_ids, warm_in, sel_err, sel_tol):
+    """Shared prologue of a scan pass: sets the device chain selection on the plan (mode 2: chain s is re-run iff
+    !(sel_err[s] <= sel_tol)) and returns (transition struct, number of listed chains, warm_in pointer, warm_in
+    stride); warm_in is one [2,K] vector shared by all chains (stride 0) or [n_chain,2,K] with one per chain."""
     if mode == 2:
         if sel_err is None or sel_err.numel() < plan.n_chain:
             raise ValueError("mode 2 needs one seam error per chain")
         plan.sel_err, plan.sel_tol = sel_err.data_ptr(), float(sel_tol)
     else:
         plan.sel_err, plan.sel_tol = None, 0.0
-
-
-def _warm(warm_in):
-    """(pointer, stride): one [2,K] vector shared by all chains, or [n_chain,2,K] with one per chain."""
+    n_ids = int(chain_ids.numel()) if chain_ids is not None else 0
     if warm_in is None:
-        return None, 0
-    return _p(warm_in), (0 if warm_in.dim() == 2 else warm_in.stride(0))
+        return op.cstruct(), n_ids, None, 0
+    return op.cstruct(), n_ids, _p(warm_in), (0 if warm_in.dim() == 2 else warm_in.stride(0))
 
 
 def forward(plan, op, ll, alpha, lmr, halo_state=None, carry_in=None, mode=0, chain_ids=None, warm_in=None,
             warm_out=None, sel_err=None, sel_tol=0.0, halo_max=0):
     """halo_max: upper bound of the per-chain warm-ups set with set_chain_halos (lockstep scan only)."""
     lib = _lib.load()
-    _select(plan, mode, sel_err, sel_tol)
-    tr = op.cstruct()
-    n_ids = int(chain_ids.numel()) if chain_ids is not None else 0
-    wp, ws = _warm(warm_in)
+    tr, n_ids, wp, ws = _pass_args(plan, op, mode, chain_ids, warm_in, sel_err, sel_tol)
     dense = getattr(op, "dense", None)
     if mode == 0 and dense is not None:
         wk = dense.workspace(plan.n_chain, ll.device)
@@ -579,10 +575,7 @@ def backward(plan, op, ll, alpha, gamma=None, gamma_lat=None, dyn_marg=None, r_o
     """xi16: optional bf16 [4, T, 2K] (alpha hi, alpha lo, r hi, r lo) that receives the operands of the
     transition-count GEMM as pieces instead of ``r_out`` (see xi16_supported)."""
     lib = _lib.load()
-    _select(plan, mode, sel_err, sel_tol)
-    tr = op.cstruct()
-    n_ids = int(chain_ids.numel()) if chain_ids is not None else 0
-    wp, ws = _warm(warm_in)
+    tr, n_ids, wp, ws = _pass_args(plan, op, mode, chain_ids, warm_in, sel_err, sel_tol)
     dense = getattr(op, "dense", None)
     if xi16 is not None:
         if r_out is not None or xi16.dtype != torch.bfloat16 or xi16.dim() != 3 or xi16.shape[0] != 4:
@@ -624,10 +617,7 @@ def viterbi_forward(plan, op, ll, bp, lmr, halo_state=None, end_msg=None, carry_
     lib = _lib.load()
     if bp.dtype != torch.int16 or bp.dim() != 3 or bp.shape[1] != 2 or not bp.is_contiguous():
         raise ValueError("bp must be a contiguous int16 [T, 2, ldbp] tensor")
-    _select(plan, mode, sel_err, sel_tol)
-    tr = op.cstruct()
-    n_ids = int(chain_ids.numel()) if chain_ids is not None else 0
-    wp, ws = _warm(warm_in)
+    tr, n_ids, wp, ws = _pass_args(plan, op, mode, chain_ids, warm_in, sel_err, sel_tol)
     check(lib.pmg_viterbi_forward(C.byref(plan), C.byref(tr), _p(ll), ll.shape[1], _p(carry_in), wp, ws,
                                   _p(warm_out), _p(bp), bp.shape[2], _p(lmr), _p(halo_state), _p(end_msg), int(mode),
                                   _p(chain_ids), n_ids, _stream()), "pmg_viterbi_forward")
@@ -688,10 +678,7 @@ def forward_compact(plan, op, ll, ax, halo_state=None, fwd_end=None, first_out=N
                     chain_ids=None, warm_in=None, warm_out=None, sel_err=None, sel_tol=0.0):
     """Forward pass writing the compact filtered posterior ax [T, K+4] (alpha[0,:], a1s, lmr per bin)."""
     lib = _lib.load()
-    _select(plan, mode, sel_err, sel_tol)
-    tr = op.cstruct()
-    n_ids = int(chain_ids.numel()) if chain_ids is not None else 0
-    wp, ws = _warm(warm_in)
+    tr, n_ids, wp, ws = _pass_args(plan, op, mode, chain_ids, warm_in, sel_err, sel_tol)
     check(lib.pmg_forward_compact(C.byref(plan), C.byref(tr), _p(ll), ll.shape[1], _p(carry_in), wp, ws,
                                   _p(warm_out), _p(ax), ax.shape[1], _p(halo_state), _p(fwd_end), _p(first_out),
                                   int(mode), _p(chain_ids), n_ids, _stream()), "pmg_forward_compact")
@@ -702,10 +689,7 @@ def backward_compact(plan, op, ll, ax, gamma16, beta_halo=None, beta_end=None, b
                      mode=0, chain_ids=None, warm_in=None, warm_out=None, sel_err=None, sel_tol=0.0):
     """Backward pass of an EM iteration: fp16 pieces of the latent posterior (and the seam messages)."""
     lib = _lib.load()
-    _select(plan, mode, sel_err, sel_tol)
-    tr = op.cstruct()
-    n_ids = int(chain_ids.numel()) if chain_ids is not None else 0
-    wp, ws = _warm(warm_in)
+    tr, n_ids, wp, ws = _pass_args(plan, op, mode, chain_ids, warm_in, sel_err, sel_tol)
     check(lib.pmg_backward_compact(C.byref(plan), C.byref(tr), _p(ll), ll.shape[1], _p(ax), ax.shape[1],
                                    _p(beta_in), wp, ws, _p(warm_out), _p(gamma16), gamma16.shape[2],
                                    _p(beta_halo), _p(beta_end), int(mode), _p(chain_ids), n_ids,
